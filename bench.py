@@ -7,10 +7,12 @@ compatible API (`define_G_inject(config)(x, embeds)`).  N>1: the same per-GPU wo
 (tile-sharded, no collective; scaling = weak).
 
 One JSON line on stdout (rank 0).  `value` = tiles/s with inputs resident in HBM; `e2e` = the same through
-host (pinned) buffers incl. H2D of tiles+embeddings and D2H of the NIR band every step.  Both are the MEDIAN over
-timed windows of exactly --steps steps (barrier + synchronize on both sides of every window, CUDA events, max over
-ranks); windows repeat until there are at least 5 and 2 s of them, p10/p90 are reported.  A clock sampler
-(nvidia-smi) runs beside every timed loop alike.
+host (pinned) buffers incl. H2D of tiles+embeddings and D2H of the NIR band every step.  Each is timed over one
+window of exactly --steps steps after the warm-up (barrier + synchronize on both sides of the window, CUDA events,
+max over ranks).  A clock sampler (nvidia-smi) runs beside every timed loop alike.
+`--dump-outputs DIR` writes the NIR prediction of the last timed `value` step (rank 0) to DIR/nir_pred.npy (float32,
+at most 64 MB: the leading tiles of a larger batch); inputs and weights are seeded, so two builds can be compared
+output for output.
 `train` sub-record: BASELINE.json configs[3] (full Pix2Pix training step, batch 32, 256x256) and configs[4]
 (data-parallel training, batch 32 per GPU, seeded mixed 128..512 px resolutions, NCCL gradient all-reduce over
 N ranks) through `nirgan_b200.trainer.Trainer`.
@@ -42,6 +44,7 @@ WORKLOAD = ("configs[1]: SatCLIP-injected ResnetGenerator (9 blocks, ngf 64) inf
             "random embeddings per GPU per step, random-init weights")
 TRAIN_RES = (128, 192, 256, 384, 512)
 GFLOP_PER_SAMPLE_256 = 391.6          # SURVEY.md 8d: minimal training-step op count (one G forward), 256x256 tile
+DUMP_LIMIT_BYTES = 64 << 20           # --dump-outputs: leading tiles of the last step's prediction up to this size
 
 
 def peaks():
@@ -410,8 +413,8 @@ def main():
     ap.add_argument("--no-train", action="store_true", help="skip the training sub-record (configs[3] / configs[4])")
     ap.add_argument("--train-batch", type=int, default=32)
     ap.add_argument("--train-steps", type=int, default=10, help="steps per timed window of the configs[3] loop")
-    ap.add_argument("--min-windows", type=int, default=5)
-    ap.add_argument("--min-seconds", type=float, default=2.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the NIR prediction of the last timed step to DIR/nir_pred.npy (float32, <= 64 MB)")
     ap.add_argument("--settle", type=float, default=1.0,
                     help="seconds of untimed work before the first window of a loop (clock ramp); 0 under a profiler")
     ap.add_argument("--sync-calls", action="store_true",
@@ -456,15 +459,16 @@ def main():
     # slices of the previous step on the generator's own streams, so consecutive steps overlap instead of meeting at a
     # barrier on the caller's stream; a timed window ends when its last step's results are complete.
     # (--sync-calls: the plain ``net(x, e)`` call, which joins the caller's stream after every step.)
-    last_done = {"ev": []}
+    last_done = {"ev": [], "y": None}
 
     def step_resident():
         with torch.no_grad():
             if args.sync_calls:
-                return net(x, e)
-            y, done = net.forward_async(x, e)
-            last_done["ev"] = done
-            return y
+                y = net(x, e)
+            else:
+                y, done = net.forward_async(x, e)
+                last_done["ev"] = done
+            last_done["y"] = y
 
     # end-to-end: every step copies its tiles + embeddings from pinned host memory and reads the NIR band back.  The
     # copies run on their own streams (double-buffered device inputs) so that step i+1's H2D and step i-1's D2H
@@ -512,12 +516,14 @@ def main():
     clock_parts = {}
     # identical conditions for both loops: a clock sampler beside each, the same warm-up rule, the same window rule
     samplers["value"] = ClockSampler(local) if rank == 0 else None
-    w_val = tm.windows(step_resident, args.steps, args.warmup, join=join_last, min_windows=args.min_windows,
-                       min_total_s=args.min_seconds, settle_s=args.settle)
+    w_val = tm.windows(step_resident, args.steps, args.warmup, join=join_last, min_windows=1, min_total_s=0.0,
+                       settle_s=args.settle)
     clock_parts["value"] = samplers["value"].stop() if samplers["value"] else None
+    # the window ends with a device synchronize: the last step's prediction is complete
+    y_last = last_done["y"].cpu() if args.dump_outputs and rank == 0 else None
     samplers["e2e"] = ClockSampler(local) if rank == 0 else None
-    w_e2e = tm.windows(step_e2e, args.steps, args.warmup, join=join_last, min_windows=args.min_windows,
-                       min_total_s=args.min_seconds, settle_s=args.settle)
+    w_e2e = tm.windows(step_e2e, args.steps, args.warmup, join=join_last, min_windows=1, min_total_s=0.0,
+                       settle_s=args.settle)
     clock_parts["e2e"] = samplers["e2e"].stop() if samplers["e2e"] else None
     ms, ms_e2e = w_val["ms_p50"], w_e2e["ms_p50"]
     # diagnostic: the host link alone (one H2D of a step's tiles from pinned memory), to read e2e against
@@ -643,8 +649,8 @@ def main():
                    "global_batch": B * world, "tile": TILE, "parallelism": f"tile-sharded x{world}, no collective",
                    "conv_impl": args.conv, "operands": args.precision + " operands, fp32 accumulate (TMEM)",
                    "chunk": Bc, "streams": B // Bc if args.chunk <= 0 else args.streams,
-                   "timing": "median over windows of exactly `steps` steps (barrier + synchronize around each window, CUDA "
-                             "events on the launching stream, max over ranks); windows repeat until >= 5 and >= 2 s",
+                   "timing": "one window of exactly `steps` steps after the warm-up (barrier + synchronize around the "
+                             "window, CUDA events on the launching stream, max over ranks)",
                    "l2": "every layer's tensors (hundreds of MB per 32-tile slice) exceed the 126 MB L2; no explicit flush",
                    "inference_buffers_gb": runner.inference_bytes() / 1e9},
         "windows": {"value": w_val, "e2e": w_e2e},
@@ -680,6 +686,12 @@ def main():
     if not args.no_cpu_baseline:
         v, cores, sample, kind = cpu_oracle_tiles_per_sec()
         line["cpu_baseline"] = {"value": v, "unit": UNIT, "cores": cores, "kind": kind, "sample": sample}
+    if y_last is not None:
+        import numpy as np
+        tile_bytes = y_last[0].numel() * 4
+        n = min(y_last.shape[0], DUMP_LIMIT_BYTES // tile_bytes)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "nir_pred.npy"), y_last[:n].float().numpy())
     emit(line)
     if dist is not None:
         dist.destroy_process_group()

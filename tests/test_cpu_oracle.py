@@ -95,37 +95,19 @@ def test_pre_norm_bias_is_cancelled_by_instance_norm():
     assert float((y0 - y1).abs().max()) < 5e-5
 
 
-def test_oracle_matches_reference_modules_when_present():
-    """When oracle/_ref holds the reference's own modules (made by oracle/make_ref.py where /root/reference exists and
-    shipped with the snapshot), the oracle port is checked against them live -- not only against the frozen fixtures."""
-    import os
-    import sys
-    import pytest
-    import torch
-    import nirgan_oracle as O
-    sys.path.insert(0, os.path.dirname(O.__file__))
-    import make_ref
-    mods = make_ref.load()
-    if mods is None:
-        pytest.skip("oracle/_ref not present")
-    nets, inj = mods
-    from nirgan_b200.config import satclip_inject_config
-    sd = O.random_state_dict(O.generator_param_shapes(inject=True), seed=5, scale_param=1.0)
-    import contextlib
-    import io
-    with contextlib.redirect_stdout(io.StringIO()):
-        ref = inj.define_G_inject(satclip_inject_config())
-    ref.load_state_dict(sd)
-    ref.eval()
-    g = torch.Generator().manual_seed(6)
-    x, e = torch.rand(2, 3, 64, 64, generator=g), torch.randn(2, 256, generator=g)
+def test_oracle_matches_reference_modules_when_present(golden_dir):
+    """The oracle port against the outputs of the reference's own define_G_inject / define_D modules (stored in
+    tests/golden by oracle/pin_against_reference.py) at 5e-6, four times tighter than the fixture tests above: the
+    SatCLIP-injected generator with scale 1.0 and the PatchGAN discriminator with non-zero biases."""
+    g = np.load(f"{golden_dir}/g_inject_64_s1.0.npz")
+    sd = _sd(O.generator_param_shapes(inject=True), g)
+    sd["scale_param"] = torch.tensor(float(g["scale"]))
     with torch.no_grad():
-        want = ref(x, e)
-        got = O.resnet_generator_forward(sd, x, embeds=e)
-    assert float((got - want).abs().max()) <= 5e-6
-    sdd = O.random_state_dict(O.discriminator_param_shapes(), seed=7, bias_std=0.1)
-    netD = nets.define_D(4, 64, "basic", 3, "instance", "normal", 0.02)
-    netD.load_state_dict(sdd)
-    xd = torch.rand(2, 4, 64, 64, generator=g)
+        got = O.resnet_generator_forward(sd, torch.from_numpy(g["x"]), embeds=torch.from_numpy(g["embeds"]))
+    assert float((got - torch.from_numpy(g["y"])).abs().max()) <= 5e-6
+    gd = np.load(f"{golden_dir}/d_64.npz")
+    assert float(gd["bias_std"]) > 0
+    sdd = _sd(O.discriminator_param_shapes(), gd)
     with torch.no_grad():
-        assert float((O.patchgan_forward(sdd, xd) - netD(xd)).abs().max()) <= 5e-6
+        got = O.patchgan_forward(sdd, torch.from_numpy(gd["x"]))
+    assert float((got - torch.from_numpy(gd["y"])).abs().max()) <= 5e-6

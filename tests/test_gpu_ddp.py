@@ -1,7 +1,7 @@
 """Multi-rank GPU parity of the data-parallel training step (BASELINE.json configs[4]; SURVEY.md 8d "config 5"):
 N ranks through NCCL, each on its shard of the batch, end with the gradients of the single-rank run on the concatenated
 batch (per-sample InstanceNorm; every loss is a mean over equal-sized shards, so averaging the shard gradients commutes).
-Needs >= 2 GPUs in the box (`gpurun --gpus 2`); skipped on a single-GPU box."""
+Needs >= 2 GPUs in the machine; skipped on a single-GPU machine."""
 import os
 import socket
 import tempfile
@@ -77,7 +77,7 @@ def _worker(rank, world, port, precision, impl, size, out_dir):
 @pytest.mark.parametrize("precision,impl,tol", [("fp32", "simt", 2e-3), ("fp16", "tc", 3e-2)], ids=["fp32-verify", "fp16-tc"])
 def test_two_rank_nccl_step_equals_single_rank_on_concatenated_batch(precision, impl, tol):
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs (gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     import torch.multiprocessing as mp
     world, size = 2, 64
     with tempfile.TemporaryDirectory() as d:
