@@ -48,6 +48,9 @@
  *   ng_image_metrics   utils/calculate_metrics.py:6-37 (L1, L2, PSNR, SSIM)
  *   ng_resize_plane / ng_hist_match / ng_sort_segments
  *                      F.interpolate + skimage.exposure.match_histograms, create_synthetic_dataset.py:34-52,111-118
+ *   ng_scene_tiles / ng_scene_blend
+ *                      the per-tile `model(hr)` loop of create_synthetic_dataset.py:100-118 over pre-cut files plus the
+ *                      cutting and stitching a user writes around it for a whole scene (the reference has neither)
  *   ng_satclip_encode  SatClIP_wrapper.predict model/satclip/satclip_wrapper.py:29-34 (location_encoder.py:73-151,
  *                      267-275; positional_encoding/spherical_harmonics.py:27-42)
  *   ng_grad_scale_pow2 / ng_unpack_weight_grad* / ng_grad_to_nchw / ng_inject_bwd / ng_nonfinite_flag
@@ -64,8 +67,8 @@ extern "C" {
 
 #define NG_VERSION 102
 
-/* element types */
-enum { NG_F32 = 0, NG_F16 = 1, NG_BF16 = 2 };
+/* element types (NG_U16: unsigned 16-bit digital numbers, scene input of ng_scene_tiles only) */
+enum { NG_F32 = 0, NG_F16 = 1, NG_BF16 = 2, NG_U16 = 3 };
 /* conv implementations */
 enum { NG_IMPL_SIMT = 0,   /* CUDA-core fp32-accumulate implicit GEMM (verification mode, any dtype) */
        NG_IMPL_TC = 1 };   /* tcgen05 / TMEM / TMA implicit GEMM (f16 or bf16 operands) */
@@ -350,6 +353,24 @@ int ng_hist_match(const float* image, const float* reference, int32_t B, int32_t
  * workspace >= segs*n*8 + segs*ceil(n/4096)*1024 bytes */
 int ng_sort_segments(const float* src, int32_t segs, int32_t n, float* sorted_out, void* workspace,
                      int64_t workspace_bytes, void* stream);
+
+/* ---- whole-scene inference (nirgan_b200/scene.py) ------------------------------------------------------------------ */
+/* Cut n windows of T x T out of a scene into the generator's input layout: scene [C][rows][W] holds scene rows
+ * [row0, row0 + rows) (a band may be resident instead of the whole scene) as NG_F32 reflectance or NG_U16 digital
+ * numbers, origins [n][2] int32 (device, 8-byte aligned) the windows' (y0, x0) in scene coordinates, dst [n][C][T][T]
+ * fp32 (16-byte aligned when T % 4 == 0).  NG_U16 values become (float)dn / dn_scale (IEEE division); a window that is
+ * not inside the resident rows is written as NaN.  One pass: conversion and cut. */
+int ng_scene_tiles(const void* scene, int32_t dtype, int32_t C, int32_t rows, int32_t W, int32_t row0,
+                   const int32_t* origins, int32_t n, int32_t T, float dn_scale, float* dst, void* stream);
+/* Weighted blend of a grid of tile predictions into output rows [y0, y1) of a W-wide band: pred [ny*nx][T][T] fp32 is
+ * the prediction of the tile at (oy[ky], ox[kx]) at index ky*nx + kx; oy [ny] and ox [nx] (device int32, ascending)
+ * must cover rows [y0, y1) and columns [0, W).  out [y1-y0][W] fp32 =
+ *   sum_t w_t p_t / sum_t w_t  over the covering tiles in ascending (ky, kx) order, fp32,
+ *   w(i, j) = w1(i) w1(j),  w1(i) = min(i + 1, T - i, overlap + 1) / (overlap + 1)
+ * (evaluated as the exact integers (overlap + 1)^2 w, the factor cancels), and exactly p_t where a single tile covers the pixel; an uncovered pixel is NaN.  Every pixel is written once (gather
+ * form, no atomics): deterministic, and bit-identical whichever band computes it. */
+int ng_scene_blend(const float* pred, const int32_t* oy, int32_t ny, const int32_t* ox, int32_t nx, int32_t T,
+                   int32_t overlap, int32_t W, int32_t y0, int32_t y1, float* out, void* stream);
 
 /* Optional generator losses (utils/losses.py:10-29 ssim_loss, :64-78 emd_loss -- pix2pix.py:12-13,233-242), forward and
  * d/dpred (dpred may be NULL).  ssim_loss: out1[0] = 1 - mean(kornia.metrics.ssim(pred, target, window)); planes = B*C;

@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "csrc", "libnirgan_b200.so")
 
 # enums of include/nirgan_b200.h
-F32, F16, BF16 = 0, 1, 2
+F32, F16, BF16, U16 = 0, 1, 2, 3
 IMPL_SIMT, IMPL_TC = 0, 1
 FORM_GATHER, FORM_PHASED, FORM_PHASED_MERGED = 0, 1, 2
 EPI_RAW, EPI_BIAS_ACT, EPI_HEAD = 0, 1, 2
@@ -81,6 +81,8 @@ _SIGNATURES = {
     "ng_ssim_loss_scratch_floats": (c_i64, [c_i32, c_i32, c_i32]),
     "ng_ssim_loss": (c_i32, [c_vp, c_vp, c_i32, c_i32, c_i32, c_i32, c_f32, c_vp, c_vp, c_vp, c_vp]),
     "ng_emd_loss": (c_i32, [c_vp, c_vp, c_i32, c_i32, c_vp, c_vp, c_vp, c_vp]),
+    "ng_scene_tiles": (c_i32, [c_vp, c_i32, c_i32, c_i32, c_i32, c_i32, c_vp, c_i32, c_i32, c_f32, c_vp, c_vp]),
+    "ng_scene_blend": (c_i32, [c_vp, c_vp, c_i32, c_vp, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_vp, c_vp]),
     "ng_satclip_encode": (c_i32, [c_vp, c_i32, c_i32, c_vp, c_i32, c_i32, c_i32, C.c_double, C.c_double, c_vp, c_vp]),
     "ng_linear": (c_i32, [c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_vp, c_vp]),
     "ng_lsgan_loss": (c_i32, [c_vp, c_i64, c_f32, c_vp, c_i32, c_vp, c_f32, c_vp]),

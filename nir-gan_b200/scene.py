@@ -1,0 +1,295 @@
+"""Whole-scene NIR prediction: overlapping tiles cut and blended on the device, sharded by row bands.
+
+The reference (and ``synth.run_shard``) only runs pre-cut tiles (create_synthetic_dataset.py:93,100-118).  Here a
+``(C, H, W)`` RGB scene -- float32 reflectance, or uint16 digital numbers read as ``dn / dn_scale`` -- becomes one
+``(1, H, W)`` NIR band:
+
+* Tile grid.  Tile ``T``, ``overlap`` in ``[0, T)``, stride ``s = T - overlap``; row origins
+  ``oy_k = min(k*s, H - T)`` for ``k = 0 .. ceil((H - T) / s)``, columns the same, tile index row-major over
+  ``(k_y, k_x)`` (``scene_tiles``).  Every pixel is covered; the last tile of a row / column is clamped to the border.
+* Per tile, exactly ``model(tile[None])`` (``Px2Px`` in eval mode, its reflect pad / crop wrapper included).  A tile's
+  bits do not depend on its batch slot or rank, so every tile of the scene loop is bit-identical to that single call.
+* Blend.  ``out(y, x) = sum_t w_t p_t / sum_t w_t`` over the covering tiles, ``w(i, j) = w1(i) w1(j)``,
+  ``w1(i) = min(1, (i + 1) / (overlap + 1), (T - i) / (overlap + 1))``; fp32 sums in ascending ``(k_y, k_x)`` order
+  (deterministic); a pixel covered by one tile gets that tile's value exactly.
+* Several GPUs: output rows are split into ``world`` contiguous bands balanced to within one row (``band_rows``).  A
+  rank computes every tile whose rows meet its band and blends only its band; tiles at band edges are computed by both
+  neighbours, with the same bits, so the assembled bands (``assemble_bands`` / ``gather_bands``) equal the ``world = 1``
+  result bit for bit.  No collective on the data path.
+
+Cutting (``ng_scene_tiles``: conversion + cut in one pass) and blending (``ng_scene_blend``: gather form, every pixel
+written once) are CUDA kernels of ``csrc/scene.cu``; the generator runs through ``Px2Px.forward_async``.  A host scene
+is copied to the device one tile row at a time on a copy stream (through pinned staging when it is not pinned itself),
+so the copy overlaps the generator.
+"""
+from __future__ import annotations
+
+from typing import Dict, List, Optional, Sequence, Tuple
+
+import torch
+
+from . import _lib as L
+
+
+def _check_grid(H: int, W: int, T: int, overlap: int) -> None:
+    if T <= 0:
+        raise ValueError(f"tile size must be positive, got {T}")
+    if not 0 <= overlap < T:
+        raise ValueError(f"overlap must lie in [0, {T}) for tile {T}, got {overlap}")
+    if H < T or W < T:
+        raise ValueError(f"scene {H}x{W} is smaller than the tile {T}x{T}")
+
+
+def _axis_origins(n: int, T: int, overlap: int) -> List[int]:
+    s = T - overlap
+    return [min(k * s, n - T) for k in range(-(-(n - T) // s) + 1)]
+
+
+def scene_grid(H: int, W: int, T: int, overlap: int) -> Tuple[List[int], List[int]]:
+    """Row origins and column origins of the tile grid (see the module docstring)."""
+    _check_grid(H, W, T, overlap)
+    return _axis_origins(H, T, overlap), _axis_origins(W, T, overlap)
+
+
+def scene_tiles(H: int, W: int, T: int, overlap: int) -> List[Tuple[int, int]]:
+    """``(y0, x0)`` of every tile in tile-index order (row-major over ``(k_y, k_x)``); e.g. to compute per-tile lon/lat
+    for the SatCLIP encoder of an injected generator."""
+    ys, xs = scene_grid(H, W, T, overlap)
+    return [(y, x) for y in ys for x in xs]
+
+
+def band_rows(H: int, rank: int, world: int) -> Tuple[int, int]:
+    """Output rows ``[y0, y1)`` of ``rank``'s band: ``world`` contiguous bands balanced to within one row."""
+    if not 1 <= world <= H:
+        raise ValueError(f"world must lie in [1, {H}] for a scene of {H} rows, got {world}")
+    if not 0 <= rank < world:
+        raise ValueError(f"rank {rank} out of range for world {world}")
+    base, extra = divmod(H, world)
+    y0 = rank * base + min(rank, extra)
+    return y0, y0 + base + (1 if rank < extra else 0)
+
+
+def band_tile_rows(row_origins: Sequence[int], T: int, y0: int, y1: int) -> Tuple[int, int]:
+    """``[k0, k1)``: the tile rows whose rows meet ``[y0, y1)`` (the origins are ascending)."""
+    ks = [k for k, o in enumerate(row_origins) if o < y1 and o + T > y0]
+    return ks[0], ks[-1] + 1
+
+
+def _padding(model) -> int:
+    d = model.config.Data
+    return d.padding_amount if d.padding else 0
+
+
+def _stream(s) -> int:
+    return s.cuda_stream
+
+
+class _HostRows:
+    """Copies scene rows ``[r_lo, r_hi)`` of a host scene to a device buffer, a chunk per tile row, on a copy stream;
+    ``ensure(k)`` issues every chunk up to tile row ``k`` and returns the event after which its rows are resident."""
+
+    def __init__(self, scene: torch.Tensor, ys: Sequence[int], k0: int, k1: int, T: int, device):
+        self.scene, self.ys, self.T, self.k1 = scene, ys, T, k1
+        C, _, W = scene.shape
+        self.r_lo = ys[k0]
+        self.dev = torch.empty(C, ys[k1 - 1] + T - self.r_lo, W, dtype=scene.dtype, device=device)
+        self.stream = torch.cuda.Stream(device)
+        self.stream.wait_stream(torch.cuda.current_stream(device))    # the buffer comes from the caller's stream
+        self.events: Dict[int, torch.cuda.Event] = {}
+        self.next_k, self.have = k0, self.r_lo
+        self.staging = []
+        if not scene.is_pinned():
+            # two pinned chunks of at most T rows: the host fills one while the other is being copied
+            self.staging = [[torch.empty(C, T, W, dtype=scene.dtype).pin_memory(), None] for _ in range(2)]
+        self.n_chunks = 0
+
+    def ensure(self, k: int) -> torch.cuda.Event:
+        while self.next_k <= min(k, self.k1 - 1):
+            a, b = self.have, self.ys[self.next_k] + self.T
+            if b > a:
+                self._copy(a, b)
+            ev = torch.cuda.Event()
+            ev.record(self.stream)
+            self.events[self.next_k] = ev
+            self.have = max(self.have, b)
+            self.next_k += 1
+        return self.events[min(k, self.k1 - 1)]
+
+    def _copy(self, a: int, b: int) -> None:
+        dst = self.dev[:, a - self.r_lo:b - self.r_lo]
+        if self.staging:
+            slot = self.staging[self.n_chunks % 2]
+            if slot[1] is not None:
+                slot[1].synchronize()                 # its previous chunk has left for the device
+            src = slot[0][:, :b - a]
+            src.copy_(self.scene[:, a:b])
+        else:
+            src = self.scene[:, a:b]
+        with torch.cuda.stream(self.stream):
+            for c in range(dst.shape[0]):             # one contiguous run of rows per channel: plain async copies
+                dst[c].copy_(src[c], non_blocking=True)
+            if self.staging:
+                done = torch.cuda.Event()
+                done.record(self.stream)
+                slot[1] = done
+        self.n_chunks += 1
+
+
+def _as_scene(scene) -> torch.Tensor:
+    if not isinstance(scene, torch.Tensor):
+        import numpy as np
+        scene = torch.from_numpy(np.ascontiguousarray(scene))
+    if scene.dim() != 3:
+        raise ValueError(f"scene must be (C, H, W), got shape {tuple(scene.shape)}")
+    if scene.dtype not in (torch.float32, torch.uint16):
+        raise ValueError(f"scene must be float32 reflectance or uint16 digital numbers, got {scene.dtype}")
+    return scene.contiguous()
+
+
+@torch.no_grad()
+def _scene_predictions(model, scene, tile: int = 256, overlap: int = 32, batch_size: int = 64,
+                       embeds: Optional[torch.Tensor] = None, dn_scale: float = 10000.0, rank: int = 0, world: int = 1):
+    """Per-tile predictions of ``rank``'s tiles.  Returns ``(pred, ys, xs, (k0, k1), (y0, y1), done, stream)``:
+    ``pred`` ``[(k1 - k0) * len(xs) (+ tail padding)][T][T]`` fp32 holds tile ``(k_y, k_x)`` at
+    ``(k_y - k0) * len(xs) + k_x`` and is complete on ``stream`` and after the event ``done``."""
+    if getattr(model, "concat", False):
+        raise NotImplementedError("predict_scene: concat-style SatCLIP generators are not supported")
+    if model.training:
+        raise RuntimeError("predict_scene: the model is in training mode, call model.eval() first")
+    inject = bool(getattr(model, "inject", False))
+    T = int(tile)
+    scene = _as_scene(scene)
+    C, H, W = scene.shape
+    ys, xs = scene_grid(H, W, T, overlap)
+    cin = model.opt.input_nc
+    if C != cin:
+        raise ValueError(f"scene has {C} channels, the model takes input_nc = {cin}")
+    pad = _padding(model)
+    if (T + 2 * pad) % 4:
+        raise ValueError(f"tile {T} with the wrapper's reflect pad {pad} gives {T + 2 * pad} rows, which the generator "
+                         f"refuses (must be divisible by 4)")
+    if batch_size < 1:
+        raise ValueError("batch_size must be >= 1")
+    if scene.dtype == torch.uint16 and not dn_scale > 0:
+        raise ValueError("dn_scale must be positive")
+    n_all = len(ys) * len(xs)
+    if inject:
+        if embeds is None:
+            raise ValueError("predict_scene: a SatCLIP-injected generator needs embeds of shape (n_tiles, 256) in "
+                             "tile-index order (scene_tiles gives the origins)")
+        if tuple(embeds.shape) != (n_all, 256):
+            raise ValueError(f"embeds must have shape ({n_all}, 256), got {tuple(embeds.shape)}")
+    elif embeds is not None:
+        raise ValueError("predict_scene: embeds given for a generator without SatCLIP injection")
+    device = next(model.parameters()).device
+    if device.type != "cuda":
+        raise RuntimeError("predict_scene: the model must be on a CUDA device (there is no CPU fallback)")
+    if scene.is_cuda and scene.device != device:
+        raise ValueError(f"scene is on {scene.device}, the model on {device}")
+
+    y0, y1 = band_rows(H, rank, world)
+    k0, k1 = band_tile_rows(ys, T, y0, y1)
+    nx = len(xs)
+    n = (k1 - k0) * nx
+    nb = -(-n // batch_size)
+    # tail padding: the last window is repeated so that every batch has batch_size tiles (one plan shape per scene)
+    local = [(ys[k], x) for k in range(k0, k1) for x in xs]
+    local += [local[-1]] * (nb * batch_size - n)
+    origins = torch.tensor(local, dtype=torch.int32).to(device, non_blocking=False)
+    emb = None
+    if inject:
+        idx = torch.arange(k0 * nx, k1 * nx)
+        idx = torch.cat([idx, idx[-1:].expand(nb * batch_size - n)])
+        emb = embeds.detach().to(device=device, dtype=torch.float32)[idx.to(device)].contiguous()
+
+    main = torch.cuda.current_stream(device)
+    cut, gather = torch.cuda.Stream(device), torch.cuda.Stream(device)
+    raw = scene.view(torch.int16) if scene.dtype == torch.uint16 else scene      # copies move the raw 16-bit words
+    host = None
+    if scene.is_cuda:
+        src, row0 = raw, 0
+    else:
+        host = _HostRows(raw, ys, k0, k1, T, device)
+        src, row0 = host.dev, host.r_lo
+    dtype = L.U16 if scene.dtype == torch.uint16 else L.F32
+    rows = src.shape[1]
+    pred = torch.empty(nb * batch_size, T, T, dtype=torch.float32, device=device)
+    cut.wait_stream(main)                 # origins / embeddings / a device scene were produced on the caller's stream
+    gather.wait_stream(main)
+    for b in range(nb):
+        lo = b * batch_size
+        with torch.cuda.stream(cut):
+            if host is not None:
+                last = min(n, lo + batch_size) - 1
+                cut.wait_event(host.ensure(last // nx + k0))
+                host.ensure(last // nx + k0 + 1)      # keep the next tile row's copy in flight
+            x = torch.empty(batch_size, C, T, T, dtype=torch.float32, device=device)
+            L.call("ng_scene_tiles", src.data_ptr(), dtype, C, rows, W, row0, origins[lo].data_ptr(), batch_size, T,
+                   float(dn_scale), x.data_ptr(), _stream(cut))
+            ready = torch.cuda.Event()
+            ready.record(cut)
+        out, done = model.forward_async(x, emb[lo:lo + batch_size] if inject else None, ready)
+        with torch.cuda.stream(gather):
+            for ev in done:
+                gather.wait_event(ev)
+            out.record_stream(gather)
+            pred[lo:lo + batch_size].copy_(out.view(batch_size, T, T))
+    origins.record_stream(cut)
+    if host is not None:
+        src.record_stream(cut)
+    fin = torch.cuda.Event()
+    fin.record(gather)
+    return pred, ys, xs, (k0, k1), (y0, y1), fin, gather
+
+
+@torch.no_grad()
+def predict_scene(model, scene, tile: int = 256, overlap: int = 32, batch_size: int = 64,
+                  embeds: Optional[torch.Tensor] = None, dn_scale: float = 10000.0, rank: int = 0, world: int = 1):
+    """NIR band of a whole scene (module docstring: grid, blend, bands).
+
+    ``model``: a ``Px2Px`` in eval mode on a CUDA device (plain or SatCLIP-injected; for the latter ``embeds`` is
+    ``(n_tiles, 256)`` in tile-index order).  ``scene``: ``(C, H, W)`` float32 reflectance or uint16 digital numbers
+    (read as ``dn / dn_scale``), host or device, ``C = input_nc``.  ``batch_size`` tiles per generator call.
+    Returns the ``(1, H, W)`` float32 device tensor for ``world = 1``, else ``(y0, y1, band)`` with ``band`` the
+    ``(1, y1 - y0, W)`` rows of this rank (``gather_bands`` / ``assemble_bands`` put the bands together).  The result
+    is valid on the caller's current stream."""
+    pred, ys, xs, (k0, k1), (y0, y1), fin, gather = _scene_predictions(
+        model, scene, tile, overlap, batch_size, embeds, dn_scale, rank, world)
+    device = pred.device
+    W = xs[-1] + tile
+    main = torch.cuda.current_stream(device)
+    band = torch.empty(1, y1 - y0, W, dtype=torch.float32, device=device)
+    with torch.cuda.stream(gather):
+        oy = torch.tensor(ys[k0:k1], dtype=torch.int32).to(device)
+        ox = torch.tensor(xs, dtype=torch.int32).to(device)
+        band.record_stream(gather)
+        L.call("ng_scene_blend", pred.data_ptr(), oy.data_ptr(), k1 - k0, ox.data_ptr(), len(xs), tile, overlap, W,
+               y0, y1, band.data_ptr(), _stream(gather))
+    main.wait_stream(gather)
+    if world == 1:
+        return band
+    return y0, y1, band
+
+
+def assemble_bands(parts: Sequence[Tuple[int, int, torch.Tensor]]) -> torch.Tensor:
+    """``(1, H, W)`` CPU tensor from the ``(y0, y1, band)`` of every rank; the bands must tile ``[0, H)`` exactly."""
+    parts = sorted(parts, key=lambda p: p[0])
+    at = 0
+    for y0, y1, band in parts:
+        if y0 != at or y1 <= y0 or band.shape[-2] != y1 - y0:
+            raise ValueError(f"bands do not tile the scene's rows: expected one starting at row {at}, got [{y0}, {y1})")
+        at = y1
+    return torch.cat([band.detach().cpu() for _, _, band in parts], dim=-2)
+
+
+def gather_bands(local: Tuple[int, int, torch.Tensor], group=None) -> torch.Tensor:
+    """Host-side assembly of the per-rank bands (the only cross-rank step; not on the GPU data path), like
+    ``synth.gather_shards``: with ``torch.distributed`` initialised every rank receives the whole ``(1, H, W)`` scene."""
+    import torch.distributed as dist
+    y0, y1, band = local
+    mine = (y0, y1, band.detach().cpu())
+    if not dist.is_available() or not dist.is_initialized() or dist.get_world_size(group) == 1:
+        return assemble_bands([mine])
+    parts = [None] * dist.get_world_size(group)
+    dist.all_gather_object(parts, mine, group=group)
+    return assemble_bands(parts)

@@ -1,0 +1,180 @@
+#!/usr/bin/env python
+"""Whole-scene prediction rate (nirgan_b200.scene.predict_scene) next to bench.py's tile rate, in one run.
+
+Workload: a seeded synthetic 8192 x 8192 uint16 scene (3 bands of digital numbers) in pinned host memory, tile 256,
+overlap 32 (37 x 37 = 1369 tiles), batch 64, the SatCLIP-injected generator of BASELINE.json configs[1] behind the Px2Px
+pad-10 wrapper (random init, per-tile random embeddings).  After --warmup scenes, --scenes scenes are timed as one
+window ending in a device synchronise.  Reported besides: the generator alone on resident 256 x 256 tiles with the same
+wrapper (where the scene loop's time goes), ng_scene_tiles / ng_scene_blend kernel times from CUDA events with their
+algorithmic bytes against a device-to-device copy measured in the same run, the card's name, power limit and clocks,
+and the `value` of `bench.py --steps K` run right after.
+
+    python tools/bench_scene.py --out profiles/scene_bench.json
+"""
+from __future__ import annotations
+
+import argparse
+import json
+import os
+import subprocess
+import sys
+import time
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")
+import torch  # noqa: E402
+
+
+def gpu_info():
+    q = "name,power.limit,clocks.sm,clocks.max.sm"
+    try:
+        out = subprocess.run(["nvidia-smi", "-i", "0", f"--query-gpu={q}", "--format=csv,noheader,nounits"],
+                             capture_output=True, text=True, timeout=30).stdout.strip()
+        f = [x.strip() for x in out.splitlines()[0].split(",")]
+        return {"name": f[0], "power_limit_w": float(f[1]), "sm_mhz": float(f[2]), "sm_max_mhz": float(f[3])}
+    except Exception as e:                          # the numbers below are still valid, only unlabeled
+        return {"error": repr(e)}
+
+
+def event_ms(fn, reps):
+    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    fn()
+    torch.cuda.synchronize()
+    a.record()
+    for _ in range(reps):
+        fn()
+    b.record()
+    torch.cuda.synchronize()
+    return a.elapsed_time(b) / reps
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--size", type=int, default=8192)
+    ap.add_argument("--tile", type=int, default=256)
+    ap.add_argument("--overlap", type=int, default=32)
+    ap.add_argument("--batch", type=int, default=64)
+    ap.add_argument("--scenes", type=int, default=4)
+    ap.add_argument("--warmup", type=int, default=1)
+    ap.add_argument("--bench-steps", type=int, default=20)
+    ap.add_argument("--out", default=None)
+    args = ap.parse_args()
+    if not torch.cuda.is_available():
+        raise SystemExit("bench_scene.py: no CUDA device")
+    import nirgan_b200  # noqa: F401
+    from nirgan_b200 import _lib as L
+    from nirgan_b200 import scene as S
+    from nirgan_b200.config import satclip_inject_config
+    from nirgan_b200.model.pix2pix import Px2Px
+
+    dev = torch.device("cuda", 0)
+    torch.manual_seed(0)
+    model = Px2Px(satclip_inject_config()).to(dev).eval()
+    model.netG.configure_b200(precision="fp16", impl="tc")
+    N, T, ov, B = args.size, args.tile, args.overlap, args.batch
+    g = torch.Generator().manual_seed(1)
+    scene = torch.randint(0, 10001, (3, N, N), generator=g, dtype=torch.int32).to(torch.int16)
+    scene = scene.view(torch.uint16).pin_memory()
+    tiles = S.scene_tiles(N, N, T, ov)
+    n = len(tiles)
+    emb = torch.randn(n, 256, generator=g)
+    padded = -(-n // B) * B
+
+    def one_scene():
+        return S.predict_scene(model, scene, tile=T, overlap=ov, batch_size=B, embeds=emb)
+
+    for _ in range(args.warmup):
+        one_scene()
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    for _ in range(args.scenes):
+        out = one_scene()
+    torch.cuda.synchronize()
+    s = (time.perf_counter() - t0) / args.scenes
+    finite = bool(torch.isfinite(out).all())
+
+    # the generator alone: resident batches of B tiles through the same wrapper (pad 10), streamed like the scene loop
+    x = torch.rand(B, 3, T, T, generator=g).to(dev)
+    e = torch.randn(B, 256, generator=g).to(dev)
+    steps = padded // B
+    last = {}
+
+    def gen_step():
+        last["y"], last["done"] = model.forward_async(x, e)
+
+    for _ in range(3):
+        gen_step()
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    for _ in range(steps * args.scenes):
+        gen_step()
+    torch.cuda.synchronize()
+    gen_tps = B * steps * args.scenes / (time.perf_counter() - t0)
+
+    # kernels on their own: one batch cut from the resident u16 scene; the blend of the whole scene
+    st = torch.cuda.current_stream().cuda_stream
+    sdev = scene.view(torch.int16).to(dev)
+    org = torch.tensor(tiles[:B], dtype=torch.int32, device=dev)
+    xb = torch.empty(B, 3, T, T, device=dev)
+    cut_ms = event_ms(lambda: L.call("ng_scene_tiles", sdev.data_ptr(), L.U16, 3, N, N, 0, org.data_ptr(), B, T,
+                                     10000.0, xb.data_ptr(), st), 50)
+    cut_bytes = B * 3 * T * T * (2 + 4)
+    ys, xs = S.scene_grid(N, N, T, ov)
+    pred = torch.rand(n, T, T, generator=torch.Generator(device=dev).manual_seed(2), device=dev) * 2 - 1
+    oy = torch.tensor(ys, dtype=torch.int32, device=dev)
+    ox = torch.tensor(xs, dtype=torch.int32, device=dev)
+    band = torch.empty(N, N, device=dev)
+    blend_ms = event_ms(lambda: L.call("ng_scene_blend", pred.data_ptr(), oy.data_ptr(), len(ys), ox.data_ptr(),
+                                       len(xs), T, ov, N, 0, N, band.data_ptr(), st), 10)
+    blend_bytes = n * T * T * 4 + N * N * 4
+    big = torch.empty(1 << 28, device=dev)                   # 1 GiB: well beyond the L2
+    big2 = torch.empty_like(big)
+    copy_ms = event_ms(lambda: big2.copy_(big), 10)
+    copy_gbs = 2 * big.numel() * 4 / copy_ms / 1e6
+    h2d_bytes = scene.numel() * 2
+    info = gpu_info()
+    del pred, band, big, big2, sdev
+    torch.cuda.empty_cache()
+
+    cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", str(args.bench_steps),
+           "--warmup", "5", "--no-train", "--no-cpu-baseline"]
+    r = subprocess.run(cmd, capture_output=True, text=True, cwd=ROOT)
+    bench_value = None
+    for line in r.stdout.splitlines():
+        if line.startswith("{"):
+            bench_value = json.loads(line).get("value")
+    tps = n / s
+    rec = {
+        "workload": f"predict_scene: {N}x{N} uint16 scene in pinned host memory, tile {T}, overlap {ov} ({n} tiles, "
+                    f"{padded} with tail padding), batch {B}, SatCLIP-injected generator behind the pad-10 wrapper, "
+                    f"fp16 / tcgen05",
+        "gpu": info,
+        "scene_s": s, "scenes_timed": args.scenes, "output_finite": finite,
+        "tiles_per_s": tps, "output_mpix_per_s": N * N / s / 1e6,
+        "generator_alone_pad10_tiles_per_s": gen_tps,
+        "tail_padding_share": (padded - n) / padded,
+        "h2d_bytes_per_scene": h2d_bytes,
+        "kernels": {
+            "copy_peak_gbs_d2d": copy_gbs,
+            "ng_scene_tiles": {"ms_per_batch": cut_ms, "bytes": cut_bytes, "gbs": cut_bytes / cut_ms / 1e6,
+                               "frac_of_copy_peak": cut_bytes / cut_ms / 1e6 / copy_gbs,
+                               "ms_per_scene": cut_ms * padded / B},
+            "ng_scene_blend": {"ms_per_scene": blend_ms, "bytes": blend_bytes, "gbs": blend_bytes / blend_ms / 1e6,
+                               "frac_of_copy_peak": blend_bytes / blend_ms / 1e6 / copy_gbs}},
+        "bench_py": {"cmd": " ".join(cmd[1:]), "value": bench_value, "returncode": r.returncode},
+        "scene_over_bench_value": tps / bench_value if bench_value else None,
+        "scene_over_generator_alone": tps / gen_tps,
+    }
+    if r.returncode != 0:
+        rec["bench_py"]["stderr_tail"] = r.stderr[-2000:]
+    txt = json.dumps(rec, indent=1)
+    print(txt)
+    if args.out:
+        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+        with open(args.out, "w") as f:
+            f.write(txt + "\n")
+
+
+if __name__ == "__main__":
+    main()
