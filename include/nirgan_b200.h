@@ -48,7 +48,7 @@
  *   ng_image_metrics   utils/calculate_metrics.py:6-37 (L1, L2, PSNR, SSIM)
  *   ng_resize_plane / ng_hist_match / ng_sort_segments
  *                      F.interpolate + skimage.exposure.match_histograms, create_synthetic_dataset.py:34-52,111-118
- *   ng_scene_tiles / ng_scene_blend
+ *   ng_scene_tiles / ng_scene_blend / ng_scene_tile_valid / ng_scene_blend_masked
  *                      the per-tile `model(hr)` loop of create_synthetic_dataset.py:100-118 over pre-cut files plus the
  *                      cutting and stitching a user writes around it for a whole scene (the reference has neither)
  *   ng_satclip_encode  SatClIP_wrapper.predict model/satclip/satclip_wrapper.py:29-34 (location_encoder.py:73-151,
@@ -371,6 +371,22 @@ int ng_scene_tiles(const void* scene, int32_t dtype, int32_t C, int32_t rows, in
  * form, no atomics): deterministic, and bit-identical whichever band computes it. */
 int ng_scene_blend(const float* pred, const int32_t* oy, int32_t ny, const int32_t* ox, int32_t nx, int32_t T,
                    int32_t overlap, int32_t W, int32_t y0, int32_t y1, float* out, void* stream);
+/* Nodata (GDAL's per-dataset mask): a pixel is nodata when every channel equals `nodata` -- NG_F32: v == nodata, and NaN
+ * matches NaN; NG_U16: the raw digital number compared as an exact float.  Valid pixels of each of n windows:
+ * scene / dtype / C / rows / W / row0 / origins as in ng_scene_tiles; counts [n] int32 (device) gets the number of
+ * valid pixels of the window, or -1 for a window not inside the resident rows.  An integer reduction without atomics
+ * (deterministic); reads C T^2 elements per window. */
+int ng_scene_tile_valid(const void* scene, int32_t dtype, int32_t C, int32_t rows, int32_t W, int32_t row0,
+                        const int32_t* origins, int32_t n, int32_t T, float nodata, int32_t* counts, void* stream);
+/* ng_scene_blend over a compacted prediction buffer, with nodata pixels written as nodata_out: tile ky*nx + kx is row
+ * slot[ky*nx + kx] (device int32) of pred, or skipped when the slot is -1 (a tile without a valid pixel; no valid pixel
+ * reads it).  scene [C][rows][W] (NG_F32 or NG_U16) holds scene rows [row0, row0 + rows), which must contain [y0, y1);
+ * a pixel that is nodata there (rule above) is nodata_out, every other pixel is exactly what ng_scene_blend gives for
+ * the uncompacted grid. */
+int ng_scene_blend_masked(const float* pred, const int32_t* slot, const int32_t* oy, int32_t ny, const int32_t* ox,
+                          int32_t nx, int32_t T, int32_t overlap, int32_t W, int32_t y0, int32_t y1, const void* scene,
+                          int32_t dtype, int32_t C, int32_t rows, int32_t row0, float nodata, float nodata_out,
+                          float* out, void* stream);
 
 /* Optional generator losses (utils/losses.py:10-29 ssim_loss, :64-78 emd_loss -- pix2pix.py:12-13,233-242), forward and
  * d/dpred (dpred may be NULL).  ssim_loss: out1[0] = 1 - mean(kornia.metrics.ssim(pred, target, window)); planes = B*C;

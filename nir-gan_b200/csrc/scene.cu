@@ -1,7 +1,11 @@
 // Whole-scene inference around the generator: cut overlapping windows of a scene into the generator's NCHW fp32 batch
 // layout, and blend the per-tile predictions back into one NIR band.  The reference only runs pre-cut tiles
-// (create_synthetic_dataset.py:93,100-118); these two kernels replace the per-tile `model(hr)` loop's hand-written
-// cutting and stitching.  Both are HBM-bound single passes; neither uses atomics, so results are bit-reproducible.
+// (create_synthetic_dataset.py:93,100-118); these kernels replace the per-tile `model(hr)` loop's hand-written
+// cutting and stitching.  All are HBM-bound single passes; none uses atomics, so results are bit-reproducible.
+//
+// Nodata (GDAL's per-dataset mask): a pixel is nodata when every channel equals the nodata value (NaN matches NaN).
+// ng_scene_tile_valid counts the valid pixels of each window so that the host can skip windows without one;
+// ng_scene_blend_masked blends a compacted prediction buffer and writes nodata pixels as a fill value.
 //
 // Blend (nirgan_b200/scene.py states the same definitions):
 //   out(y, x) = sum_t w_t(y, x) p_t(y, x) / sum_t w_t(y, x)   over the tiles t covering (y, x), ascending (k_y, k_x)
@@ -43,6 +47,62 @@ scene_tiles_kernel(const E* __restrict__ scene, int C, int rows, int W, int row0
   }
 }
 
+// v == nodata, with NaN matching NaN (so -0.0 matches 0.0); uint16 values are exact in fp32
+template <typename E> __device__ __forceinline__ bool is_nodata(E v, float nodata);
+template <> __device__ __forceinline__ bool is_nodata<float>(float v, float nodata) {
+  return v == nodata || (v != v && nodata != nodata);
+}
+template <> __device__ __forceinline__ bool is_nodata<uint16_t>(uint16_t v, float nodata) { return (float)v == nodata; }
+
+// pixel `at` of the planes scene[c * plane ..]: valid unless every channel is nodata.  All channels are read (no early
+// exit), so the loads of a thread issue together and the bytes read are C per pixel whatever the data.
+template <typename E>
+__device__ __forceinline__ bool pixel_valid(const E* __restrict__ scene, int C, size_t plane, size_t at, float nodata) {
+  bool valid = false;
+  for (int c = 0; c < C; ++c) valid |= !is_nodata<E>(scene[(size_t)c * plane + at], nodata);
+  return valid;
+}
+
+// one block per window (a host scene's launch covers one tile row, a few dozen windows: 512 threads keep more loads in
+// flight per SM than 256).  The count is a fixed-order integer reduction (warp sums, then the block's warp partials).
+constexpr int SV_THREADS = 512;
+
+template <typename E>
+__global__ void __launch_bounds__(SV_THREADS)
+scene_valid_kernel(const E* __restrict__ scene, int C, int rows, int W, int row0, const int2* __restrict__ origins,
+                   int T, float nodata, int* __restrict__ counts) {
+  const int tile = blockIdx.x;
+  const int2 o = origins[tile];                       // (y0, x0) in scene coordinates
+  const int r = o.x - row0;
+  if (!(r >= 0 && r + T <= rows && o.y >= 0 && o.y + T <= W)) {   // outside the resident rows: -1, nothing read
+    if (threadIdx.x == 0) counts[tile] = -1;
+    return;
+  }
+  const E* src = scene + (size_t)r * W + o.y;
+  const size_t plane = (size_t)rows * W;
+  int cnt = 0;
+#pragma unroll 4
+  for (int e = threadIdx.x; e < T * T; e += SV_THREADS) {
+    const int i = e / T, j = e - i * T;
+    cnt += pixel_valid<E>(src, C, plane, (size_t)i * W + j, nodata);
+  }
+  __shared__ int part[SV_THREADS / 32];
+  cnt = __reduce_add_sync(0xffffffffu, cnt);
+  if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = cnt;
+  __syncthreads();
+  if (threadIdx.x < 32) {
+    cnt = __reduce_add_sync(0xffffffffu, threadIdx.x < SV_THREADS / 32 ? part[threadIdx.x] : 0);
+    if (threadIdx.x == 0) counts[tile] = cnt;
+  }
+}
+
+// the nodata mask of the masked blend: scene rows [row0, row0 + rows) resident as scene [C][rows][W]
+template <typename E> struct SceneMask {
+  const E* scene;
+  int C, rows, row0;
+  float nodata, nodata_out;
+};
+
 // (overlap + 1) * w1(i): the common factor cancels in the normalised sum, and the integer weights and their sums are
 // exact in fp32 (at most (overlap + 1)^2 per tile)
 __device__ __forceinline__ int blend_m1(int i, int T, int ov1) { return min(min(i + 1, T - i), ov1); }
@@ -54,8 +114,12 @@ __device__ __forceinline__ int first_cover(const int* __restrict__ o, int n, int
   return lo;
 }
 
-// out(y, x) over the covering tiles: rows ky0.. of oy, columns found here (ascending (ky, kx), fp32)
-__device__ __forceinline__ float blend_pixel(const float* __restrict__ pred, const int* __restrict__ oy, int ny, int ky0,
+// out(y, x) over the covering tiles: rows ky0.. of oy, columns found here (ascending (ky, kx), fp32).  SLOT: tile
+// ky * nx + kx is row slot[ky * nx + kx] of the compacted pred, and a skipped tile (-1) is passed over; it never covers
+// a valid pixel, since a tile with a valid pixel is computed.  Without SLOT, tile ky * nx + kx is row ky * nx + kx.
+template <bool SLOT>
+__device__ __forceinline__ float blend_pixel(const float* __restrict__ pred, const int* __restrict__ slot,
+                                             const int* __restrict__ oy, int ny, int ky0,
                                              const int* __restrict__ ox, int nx, int T, int ov1, int y, int x) {
   const int kx0 = first_cover(ox, nx, T, x);
   float acc = 0.f, wsum = 0.f, last = 0.f;
@@ -67,7 +131,13 @@ __device__ __forceinline__ float blend_pixel(const float* __restrict__ pred, con
     for (int kx = kx0; kx < nx && ox[kx] <= x; ++kx) {
       const int j = x - ox[kx];
       const float w = (float)(my * blend_m1(j, T, ov1));
-      last = __ldg(prow + (size_t)kx * T * T + j);
+      if constexpr (SLOT) {
+        const int s = __ldg(slot + ky * nx + kx);
+        if (s < 0) continue;
+        last = __ldg(pred + (size_t)s * T * T + (size_t)i * T + j);
+      } else {
+        last = __ldg(prow + (size_t)kx * T * T + j);
+      }
       acc = __fmaf_rn(w, last, acc);
       wsum = __fadd_rn(wsum, w);
       ++cnt;
@@ -77,11 +147,13 @@ __device__ __forceinline__ float blend_pixel(const float* __restrict__ pred, con
 }
 
 // gather form: every output pixel of rows [y0, y0 + rows) reads its covering tiles and is written once.  V consecutive
-// pixels of one row per thread (V = 4 when W % 4 == 0: one 16-byte store).
-template <int V>
+// pixels of one row per thread (V = 4 when W % 4 == 0: one 16-byte store).  MASK: pred is compacted through slot, and
+// a nodata pixel of the resident scene rows is written as mask.nodata_out without reading any prediction.
+template <int V, bool MASK = false, typename E = float>
 __global__ void __launch_bounds__(SC_THREADS)
-scene_blend_kernel(const float* __restrict__ pred, const int* __restrict__ oy, int ny, const int* __restrict__ ox, int nx,
-                   int T, int overlap, int W, int y0, int rows, float* __restrict__ out) {
+scene_blend_kernel(const float* __restrict__ pred, const int* __restrict__ slot, const int* __restrict__ oy, int ny,
+                   const int* __restrict__ ox, int nx, int T, int overlap, int W, int y0, int rows, SceneMask<E> mask,
+                   float* __restrict__ out) {
   const int x = (blockIdx.x * blockDim.x + threadIdx.x) * V;
   if (x >= W) return;
   const int ov1 = overlap + 1;
@@ -89,14 +161,32 @@ scene_blend_kernel(const float* __restrict__ pred, const int* __restrict__ oy, i
     const int y = y0 + row;
     const int ky0 = first_cover(oy, ny, T, y);
     float* o = out + (size_t)row * W + x;
+    auto px = [&](int xx) -> float {
+      if constexpr (MASK) {
+        const E* srow = mask.scene + (size_t)(y - mask.row0) * W;
+        if (!pixel_valid<E>(srow, mask.C, (size_t)mask.rows * W, xx, mask.nodata)) return mask.nodata_out;
+      }
+      return blend_pixel<MASK>(pred, slot, oy, ny, ky0, ox, nx, T, ov1, y, xx);
+    };
     if constexpr (V == 4)
-      *reinterpret_cast<float4*>(o) = make_float4(blend_pixel(pred, oy, ny, ky0, ox, nx, T, ov1, y, x),
-                                                  blend_pixel(pred, oy, ny, ky0, ox, nx, T, ov1, y, x + 1),
-                                                  blend_pixel(pred, oy, ny, ky0, ox, nx, T, ov1, y, x + 2),
-                                                  blend_pixel(pred, oy, ny, ky0, ox, nx, T, ov1, y, x + 3));
+      *reinterpret_cast<float4*>(o) = make_float4(px(x), px(x + 1), px(x + 2), px(x + 3));
     else
-      *o = blend_pixel(pred, oy, ny, ky0, ox, nx, T, ov1, y, x);
+      *o = px(x);
   }
+}
+
+template <bool MASK, typename E>
+int launch_blend(const float* pred, const int* slot, const int* oy, int ny, const int* ox, int nx, int T, int overlap,
+                 int W, int y0, int y1, SceneMask<E> mask, float* out, void* stream) {
+  const bool vec = W % 4 == 0 && ((uintptr_t)out & 15) == 0;
+  const int V = vec ? 4 : 1;
+  const int per_row = (W + V - 1) / V;
+  const dim3 grid((per_row + SC_THREADS - 1) / SC_THREADS, y1 - y0 < 65535 ? y1 - y0 : 65535);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (vec) scene_blend_kernel<4, MASK, E><<<grid, SC_THREADS, 0, st>>>(pred, slot, oy, ny, ox, nx, T, overlap, W, y0, y1 - y0, mask, out);
+  else scene_blend_kernel<1, MASK, E><<<grid, SC_THREADS, 0, st>>>(pred, slot, oy, ny, ox, nx, T, overlap, W, y0, y1 - y0, mask, out);
+  NG_LAUNCH_CHECK("scene_blend_kernel");
+  return NG_OK;
 }
 
 }  // namespace ng
@@ -130,19 +220,54 @@ extern "C" int ng_scene_tiles(const void* scene, int32_t dtype, int32_t C, int32
   return NG_OK;
 }
 
-extern "C" int ng_scene_blend(const float* pred, const int32_t* oy, int32_t ny, const int32_t* ox, int32_t nx, int32_t T,
-                              int32_t overlap, int32_t W, int32_t y0, int32_t y1, float* out, void* stream) {
+extern "C" int ng_scene_tile_valid(const void* scene, int32_t dtype, int32_t C, int32_t rows, int32_t W, int32_t row0,
+                                   const int32_t* origins, int32_t n, int32_t T, float nodata, int32_t* counts,
+                                   void* stream) {
   int r = require_sm100(); if (r) return r;
+  NG_REQUIRE(scene && origins && counts && C > 0 && rows > 0 && W > 0 && row0 >= 0 && n > 0 && T > 0, NG_E_ARG,
+             "scene_tile_valid: bad arguments");
+  NG_REQUIRE(dtype == NG_F32 || dtype == NG_U16, NG_E_ARG, "scene_tile_valid: the scene must be NG_F32 or NG_U16");
+  NG_REQUIRE(((uintptr_t)origins & 7) == 0, NG_E_ALIGN, "scene_tile_valid: origins must be 8-byte aligned");
+  cudaStream_t st = (cudaStream_t)stream;
+  const int2* org = reinterpret_cast<const int2*>(origins);
+  if (dtype == NG_F32)
+    scene_valid_kernel<float><<<n, SV_THREADS, 0, st>>>((const float*)scene, C, rows, W, row0, org, T, nodata, counts);
+  else
+    scene_valid_kernel<uint16_t><<<n, SV_THREADS, 0, st>>>((const uint16_t*)scene, C, rows, W, row0, org, T, nodata, counts);
+  NG_LAUNCH_CHECK("scene_valid_kernel");
+  return NG_OK;
+}
+
+static int check_blend(const float* pred, const int32_t* oy, int32_t ny, const int32_t* ox, int32_t nx, int32_t T,
+                       int32_t overlap, int32_t W, int32_t y0, int32_t y1, float* out) {
   NG_REQUIRE(pred && oy && ox && out && ny > 0 && nx > 0 && T > 0 && W >= T && y0 >= 0 && y1 > y0, NG_E_ARG,
              "scene_blend: bad arguments");
   NG_REQUIRE(overlap >= 0 && overlap < T, NG_E_ARG, "scene_blend: overlap %d outside [0, %d)", overlap, T);
-  const bool vec = W % 4 == 0 && ((uintptr_t)out & 15) == 0;
-  const int V = vec ? 4 : 1;
-  const int per_row = (W + V - 1) / V;
-  const dim3 grid((per_row + SC_THREADS - 1) / SC_THREADS, y1 - y0 < 65535 ? y1 - y0 : 65535);
-  cudaStream_t st = (cudaStream_t)stream;
-  if (vec) scene_blend_kernel<4><<<grid, SC_THREADS, 0, st>>>(pred, oy, ny, ox, nx, T, overlap, W, y0, y1 - y0, out);
-  else scene_blend_kernel<1><<<grid, SC_THREADS, 0, st>>>(pred, oy, ny, ox, nx, T, overlap, W, y0, y1 - y0, out);
-  NG_LAUNCH_CHECK("scene_blend_kernel");
   return NG_OK;
+}
+
+extern "C" int ng_scene_blend(const float* pred, const int32_t* oy, int32_t ny, const int32_t* ox, int32_t nx, int32_t T,
+                              int32_t overlap, int32_t W, int32_t y0, int32_t y1, float* out, void* stream) {
+  int r = require_sm100(); if (r) return r;
+  r = check_blend(pred, oy, ny, ox, nx, T, overlap, W, y0, y1, out); if (r) return r;
+  return launch_blend<false, float>(pred, nullptr, oy, ny, ox, nx, T, overlap, W, y0, y1, SceneMask<float>{}, out, stream);
+}
+
+extern "C" int ng_scene_blend_masked(const float* pred, const int32_t* slot, const int32_t* oy, int32_t ny,
+                                     const int32_t* ox, int32_t nx, int32_t T, int32_t overlap, int32_t W, int32_t y0,
+                                     int32_t y1, const void* scene, int32_t dtype, int32_t C, int32_t rows,
+                                     int32_t row0, float nodata, float nodata_out, float* out, void* stream) {
+  int r = require_sm100(); if (r) return r;
+  r = check_blend(pred, oy, ny, ox, nx, T, overlap, W, y0, y1, out); if (r) return r;
+  NG_REQUIRE(slot && scene && C > 0 && rows > 0 && row0 >= 0, NG_E_ARG, "scene_blend_masked: bad arguments");
+  NG_REQUIRE(dtype == NG_F32 || dtype == NG_U16, NG_E_ARG, "scene_blend_masked: the scene must be NG_F32 or NG_U16");
+  NG_REQUIRE(row0 <= y0 && y1 <= row0 + rows, NG_E_SHAPE,
+             "scene_blend_masked: rows [%d, %d) are not inside the resident scene rows [%d, %d)", y0, y1, row0,
+             row0 + rows);
+  if (dtype == NG_F32)
+    return launch_blend<true, float>(pred, slot, oy, ny, ox, nx, T, overlap, W, y0, y1,
+                                     SceneMask<float>{(const float*)scene, C, rows, row0, nodata, nodata_out}, out, stream);
+  return launch_blend<true, uint16_t>(pred, slot, oy, ny, ox, nx, T, overlap, W, y0, y1,
+                                      SceneMask<uint16_t>{(const uint16_t*)scene, C, rows, row0, nodata, nodata_out},
+                                      out, stream);
 }

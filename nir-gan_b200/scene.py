@@ -17,14 +17,23 @@ The reference (and ``synth.run_shard``) only runs pre-cut tiles (create_syntheti
   neighbours, with the same bits, so the assembled bands (``assemble_bands`` / ``gather_bands``) equal the ``world = 1``
   result bit for bit.  No collective on the data path.
 
+* Nodata (``nodata=``, off by default).  A pixel is nodata when every channel equals ``nodata`` (GDAL's per-dataset
+  mask; NaN matches NaN; uint16 scenes compare the raw digital number).  A tile without a valid pixel is skipped: never
+  cut, never run, its ``embeds`` row never read.  Nodata pixels come out as ``nodata_out``; every valid pixel is
+  bit-identical to ``nodata=None``, because each tile covering it contains it and so is computed: the blend sees the
+  same tiles in the same order with the same weights.
+
 Cutting (``ng_scene_tiles``: conversion + cut in one pass) and blending (``ng_scene_blend``: gather form, every pixel
 written once) are CUDA kernels of ``csrc/scene.cu``; the generator runs through ``Px2Px.forward_async``.  A host scene
 is copied to the device one tile row at a time on a copy stream (through pinned staging when it is not pinned itself),
-so the copy overlaps the generator.
+so the copy overlaps the generator.  With ``nodata`` the valid pixels of each tile are counted on the device
+(``ng_scene_tile_valid``: once over a device scene, per tile row right after its copy for a host scene), the computed
+tiles are batched in tile-index order, and ``ng_scene_blend_masked`` blends the compacted predictions.
 """
 from __future__ import annotations
 
-from typing import Dict, List, Optional, Sequence, Tuple
+import numbers
+from typing import Dict, List, NamedTuple, Optional, Sequence, Tuple
 
 import torch
 
@@ -146,12 +155,81 @@ def _as_scene(scene) -> torch.Tensor:
     return scene.contiguous()
 
 
+def _nodata_value(nodata, dtype: torch.dtype) -> float:
+    """``nodata`` as the float the kernels compare with: an integer in [0, 65535] for uint16 scenes (the raw digital
+    number), any float for float32 scenes (compared in fp32)."""
+    if isinstance(nodata, bool) or not isinstance(nodata, numbers.Real):
+        raise ValueError(f"nodata must be a number, got {nodata!r}")
+    v = float(nodata)
+    if dtype == torch.uint16 and not (v.is_integer() and 0 <= v <= 65535):
+        raise ValueError(f"nodata of a uint16 scene must be an integer in [0, 65535], got {nodata!r}")
+    return v
+
+
+class _TileCounts:
+    """Valid-pixel counts (``ng_scene_tile_valid``) of the tiles of tile rows ``[k0, k1)``, local tile index
+    ``(k - k0) * nx + kx``.  A device scene is counted in one launch and read back at once; a host scene one tile row at
+    a time on the copy stream right after that row's copy, read back into pinned memory behind an event, so that
+    ``row(k)`` waits for row ``k`` only while the next row's copy is already in flight."""
+
+    def __init__(self, src, dtype, row0, origins, nx, k0, k1, T, nodata, host: Optional[_HostRows], stream):
+        self.src, self.dtype, self.row0, self.origins = src, dtype, row0, origins
+        self.nx, self.k0, self.k1, self.T, self.nodata, self.host = nx, k0, k1, T, nodata, host
+        n = (k1 - k0) * nx
+        self.dev = torch.empty(n, dtype=torch.int32, device=src.device)
+        if host is None:
+            self._launch(0, n, stream)
+            with torch.cuda.stream(stream):
+                self.counts = self.dev.cpu()
+            return
+        self.dev.record_stream(host.stream)
+        self.counts = torch.empty(n, dtype=torch.int32, pin_memory=True)
+        self.events: Dict[int, torch.cuda.Event] = {}
+        self.next_k = k0
+
+    def _launch(self, lo: int, hi: int, stream) -> None:
+        C, rows, W = self.src.shape
+        L.call("ng_scene_tile_valid", self.src.data_ptr(), self.dtype, C, rows, W, self.row0,
+               self.origins[lo].data_ptr(), hi - lo, self.T, self.nodata, self.dev[lo:].data_ptr(), _stream(stream))
+
+    def _issue(self, k: int) -> None:
+        while self.next_k <= min(k, self.k1 - 1):
+            self.host.ensure(self.next_k)             # the row's copy, then its count, on the copy stream
+            lo = (self.next_k - self.k0) * self.nx
+            hi = lo + self.nx
+            self._launch(lo, hi, self.host.stream)
+            with torch.cuda.stream(self.host.stream):
+                self.counts[lo:hi].copy_(self.dev[lo:hi], non_blocking=True)
+                ev = torch.cuda.Event()
+                ev.record(self.host.stream)
+            self.events[self.next_k] = ev
+            self.next_k += 1
+
+    def row(self, k: int) -> List[int]:
+        if self.host is not None:
+            self._issue(k + 1)                        # keep the next tile row's copy in flight
+            self.events[k].synchronize()
+        lo = (k - self.k0) * self.nx
+        return self.counts[lo:lo + self.nx].tolist()
+
+
+class _Run(NamedTuple):
+    pred: torch.Tensor            # [rows][T][T] fp32, tile at its slot (every tile's own index without nodata)
+    ys: List[int]
+    xs: List[int]
+    k: Tuple[int, int]            # tile rows [k0, k1) of the band
+    band: Tuple[int, int]         # output rows [y0, y1)
+    done: torch.cuda.Event
+    stream: torch.cuda.Stream
+    slot: Optional[List[int]]     # nodata only: local tile index -> row of pred, -1 for a skipped tile
+    mask: Optional[tuple]         # nodata only: (resident scene rows, NG dtype, row0, nodata)
+
+
 @torch.no_grad()
-def _scene_predictions(model, scene, tile: int = 256, overlap: int = 32, batch_size: int = 64,
-                       embeds: Optional[torch.Tensor] = None, dn_scale: float = 10000.0, rank: int = 0, world: int = 1):
-    """Per-tile predictions of ``rank``'s tiles.  Returns ``(pred, ys, xs, (k0, k1), (y0, y1), done, stream)``:
-    ``pred`` ``[(k1 - k0) * len(xs) (+ tail padding)][T][T]`` fp32 holds tile ``(k_y, k_x)`` at
-    ``(k_y - k0) * len(xs) + k_x`` and is complete on ``stream`` and after the event ``done``."""
+def _scene_run(model, scene, tile: int, overlap: int, batch_size: int, embeds: Optional[torch.Tensor], dn_scale: float,
+               rank: int, world: int, nodata) -> _Run:
+    """Per-tile predictions of ``rank``'s computed tiles (every tile without ``nodata``), complete on ``stream`` and
+    after the event ``done``."""
     if getattr(model, "concat", False):
         raise NotImplementedError("predict_scene: concat-style SatCLIP generators are not supported")
     if model.training:
@@ -159,6 +237,7 @@ def _scene_predictions(model, scene, tile: int = 256, overlap: int = 32, batch_s
     inject = bool(getattr(model, "inject", False))
     T = int(tile)
     scene = _as_scene(scene)
+    nd = None if nodata is None else _nodata_value(nodata, scene.dtype)
     C, H, W = scene.shape
     ys, xs = scene_grid(H, W, T, overlap)
     cin = model.opt.input_nc
@@ -191,16 +270,8 @@ def _scene_predictions(model, scene, tile: int = 256, overlap: int = 32, batch_s
     k0, k1 = band_tile_rows(ys, T, y0, y1)
     nx = len(xs)
     n = (k1 - k0) * nx
-    nb = -(-n // batch_size)
-    # tail padding: the last window is repeated so that every batch has batch_size tiles (one plan shape per scene)
     local = [(ys[k], x) for k in range(k0, k1) for x in xs]
-    local += [local[-1]] * (nb * batch_size - n)
-    origins = torch.tensor(local, dtype=torch.int32).to(device, non_blocking=False)
-    emb = None
-    if inject:
-        idx = torch.arange(k0 * nx, k1 * nx)
-        idx = torch.cat([idx, idx[-1:].expand(nb * batch_size - n)])
-        emb = embeds.detach().to(device=device, dtype=torch.float32)[idx.to(device)].contiguous()
+    emb = embeds.detach().to(device=device, dtype=torch.float32) if inject else None
 
     main = torch.cuda.current_stream(device)
     cut, gather = torch.cuda.Stream(device), torch.cuda.Stream(device)
@@ -213,58 +284,136 @@ def _scene_predictions(model, scene, tile: int = 256, overlap: int = 32, batch_s
         src, row0 = host.dev, host.r_lo
     dtype = L.U16 if scene.dtype == torch.uint16 else L.F32
     rows = src.shape[1]
-    pred = torch.empty(nb * batch_size, T, T, dtype=torch.float32, device=device)
-    cut.wait_stream(main)                 # origins / embeddings / a device scene were produced on the caller's stream
+    cut.wait_stream(main)                 # embeddings / a device scene were produced on the caller's stream
     gather.wait_stream(main)
-    for b in range(nb):
-        lo = b * batch_size
+    counts = None
+    if nd is not None:
+        all_origins = torch.tensor(local, dtype=torch.int32).to(device)
+        counts = _TileCounts(src, dtype, row0, all_origins, nx, k0, k1, T, nd, host, cut)
+        all_origins.record_stream(cut if host is None else host.stream)
+    # a host scene learns its computed tiles one tile row at a time while the generator runs: its prediction buffer is
+    # sized for every tile of the band, a device scene's for the computed tiles only
+    n_pred = n if counts is None or host is not None else sum(c > 0 for c in counts.counts.tolist())
+    cap = -(-n_pred // batch_size) * batch_size
+    pred = torch.empty(max(cap, 1), T, T, dtype=torch.float32, device=device)
+    # batch b's origins (and embedding rows) at [b * batch_size, (b + 1) * batch_size): pinned, then one async copy
+    org_h = torch.empty(max(cap, 1), 2, dtype=torch.int32, pin_memory=True)
+    org = torch.empty_like(org_h, device=device)
+    idx_h = torch.empty(max(cap, 1), dtype=torch.int64, pin_memory=True) if inject else None
+    idx = torch.empty_like(idx_h, device=device) if inject else None
+    slot = [-1] * n if nd is not None else None
+    nb = 0
+
+    def run(tiles: List[int]) -> None:
+        nonlocal nb
+        lo = nb * batch_size
+        # tail padding: the last computed window is repeated so that every batch has batch_size tiles (one plan shape)
+        tiles = tiles + [tiles[-1]] * (batch_size - len(tiles))
+        org_h[lo:lo + batch_size] = torch.tensor([local[t] for t in tiles], dtype=torch.int32)
+        if inject:
+            idx_h[lo:lo + batch_size] = torch.tensor(tiles, dtype=torch.int64) + k0 * nx
         with torch.cuda.stream(cut):
             if host is not None:
-                last = min(n, lo + batch_size) - 1
-                cut.wait_event(host.ensure(last // nx + k0))
-                host.ensure(last // nx + k0 + 1)      # keep the next tile row's copy in flight
+                last = tiles[-1] // nx + k0
+                cut.wait_event(host.ensure(last))
+                host.ensure(last + 1)                 # keep the next tile row's copy in flight
+            org[lo:lo + batch_size].copy_(org_h[lo:lo + batch_size], non_blocking=True)
             x = torch.empty(batch_size, C, T, T, dtype=torch.float32, device=device)
-            L.call("ng_scene_tiles", src.data_ptr(), dtype, C, rows, W, row0, origins[lo].data_ptr(), batch_size, T,
+            L.call("ng_scene_tiles", src.data_ptr(), dtype, C, rows, W, row0, org[lo].data_ptr(), batch_size, T,
                    float(dn_scale), x.data_ptr(), _stream(cut))
+            e = None
+            if inject:
+                idx[lo:lo + batch_size].copy_(idx_h[lo:lo + batch_size], non_blocking=True)
+                e = emb.index_select(0, idx[lo:lo + batch_size])
             ready = torch.cuda.Event()
             ready.record(cut)
-        out, done = model.forward_async(x, emb[lo:lo + batch_size] if inject else None, ready)
+        out, done = model.forward_async(x, e, ready)
         with torch.cuda.stream(gather):
             for ev in done:
                 gather.wait_event(ev)
             out.record_stream(gather)
             pred[lo:lo + batch_size].copy_(out.view(batch_size, T, T))
-    origins.record_stream(cut)
+        nb += 1
+
+    # batches: consecutive runs of computed tiles in tile-index order
+    pending: List[int] = []
+    for k in range(k0, k1):
+        base = (k - k0) * nx
+        if counts is None:
+            pending += range(base, base + nx)
+        else:
+            for kx, c in enumerate(counts.row(k)):
+                if c > 0:
+                    slot[base + kx] = nb * batch_size + len(pending)
+                    pending.append(base + kx)
+        while len(pending) >= batch_size:
+            run(pending[:batch_size])
+            pending = pending[batch_size:]
+    if pending:
+        run(pending)
+    org.record_stream(cut)
+    if inject:
+        idx.record_stream(cut)
+        emb.record_stream(cut)
     if host is not None:
         src.record_stream(cut)
+    mask = None
+    if nd is not None:
+        if host is not None:
+            gather.wait_event(host.ensure(k1 - 1))    # the blend reads the mask from every resident row
+            src.record_stream(gather)
+        mask = (src, dtype, row0, nd)
     fin = torch.cuda.Event()
     fin.record(gather)
-    return pred, ys, xs, (k0, k1), (y0, y1), fin, gather
+    return _Run(pred, ys, xs, (k0, k1), (y0, y1), fin, gather, slot, mask)
+
+
+@torch.no_grad()
+def _scene_predictions(model, scene, tile: int = 256, overlap: int = 32, batch_size: int = 64,
+                       embeds: Optional[torch.Tensor] = None, dn_scale: float = 10000.0, rank: int = 0, world: int = 1):
+    """Per-tile predictions of ``rank``'s tiles.  Returns ``(pred, ys, xs, (k0, k1), (y0, y1), done, stream)``:
+    ``pred`` ``[(k1 - k0) * len(xs) (+ tail padding)][T][T]`` fp32 holds tile ``(k_y, k_x)`` at
+    ``(k_y - k0) * len(xs) + k_x`` and is complete on ``stream`` and after the event ``done``."""
+    r = _scene_run(model, scene, tile, overlap, batch_size, embeds, dn_scale, rank, world, None)
+    return r.pred, r.ys, r.xs, r.k, r.band, r.done, r.stream
 
 
 @torch.no_grad()
 def predict_scene(model, scene, tile: int = 256, overlap: int = 32, batch_size: int = 64,
-                  embeds: Optional[torch.Tensor] = None, dn_scale: float = 10000.0, rank: int = 0, world: int = 1):
-    """NIR band of a whole scene (module docstring: grid, blend, bands).
+                  embeds: Optional[torch.Tensor] = None, dn_scale: float = 10000.0, rank: int = 0, world: int = 1,
+                  nodata=None, nodata_out: float = float("nan")):
+    """NIR band of a whole scene (module docstring: grid, blend, bands, nodata).
 
     ``model``: a ``Px2Px`` in eval mode on a CUDA device (plain or SatCLIP-injected; for the latter ``embeds`` is
     ``(n_tiles, 256)`` in tile-index order).  ``scene``: ``(C, H, W)`` float32 reflectance or uint16 digital numbers
     (read as ``dn / dn_scale``), host or device, ``C = input_nc``.  ``batch_size`` tiles per generator call.
+    ``nodata``: ``None`` (every pixel holds data), or the value that marks a nodata pixel in every channel -- an integer
+    in [0, 65535] compared with the raw digital numbers of a uint16 scene, any float (NaN included) for a float32 scene.
+    Tiles without a valid pixel are skipped (their ``embeds`` rows are never read) and nodata pixels are ``nodata_out``.
     Returns the ``(1, H, W)`` float32 device tensor for ``world = 1``, else ``(y0, y1, band)`` with ``band`` the
     ``(1, y1 - y0, W)`` rows of this rank (``gather_bands`` / ``assemble_bands`` put the bands together).  The result
     is valid on the caller's current stream."""
-    pred, ys, xs, (k0, k1), (y0, y1), fin, gather = _scene_predictions(
-        model, scene, tile, overlap, batch_size, embeds, dn_scale, rank, world)
-    device = pred.device
-    W = xs[-1] + tile
+    if nodata is not None and (isinstance(nodata_out, bool) or not isinstance(nodata_out, numbers.Real)):
+        raise ValueError(f"nodata_out must be a number, got {nodata_out!r}")
+    r = _scene_run(model, scene, tile, overlap, batch_size, embeds, dn_scale, rank, world, nodata)
+    (k0, k1), (y0, y1), gather = r.k, r.band, r.stream
+    device = r.pred.device
+    W = r.xs[-1] + tile
     main = torch.cuda.current_stream(device)
     band = torch.empty(1, y1 - y0, W, dtype=torch.float32, device=device)
     with torch.cuda.stream(gather):
-        oy = torch.tensor(ys[k0:k1], dtype=torch.int32).to(device)
-        ox = torch.tensor(xs, dtype=torch.int32).to(device)
+        oy = torch.tensor(r.ys[k0:k1], dtype=torch.int32).to(device)
+        ox = torch.tensor(r.xs, dtype=torch.int32).to(device)
         band.record_stream(gather)
-        L.call("ng_scene_blend", pred.data_ptr(), oy.data_ptr(), k1 - k0, ox.data_ptr(), len(xs), tile, overlap, W,
-               y0, y1, band.data_ptr(), _stream(gather))
+        if r.mask is None:
+            L.call("ng_scene_blend", r.pred.data_ptr(), oy.data_ptr(), k1 - k0, ox.data_ptr(), len(r.xs), tile, overlap,
+                   W, y0, y1, band.data_ptr(), _stream(gather))
+        else:
+            src, dtype, row0, nd = r.mask
+            slot = torch.tensor(r.slot, dtype=torch.int32).to(device)
+            L.call("ng_scene_blend_masked", r.pred.data_ptr(), slot.data_ptr(), oy.data_ptr(), k1 - k0, ox.data_ptr(),
+                   len(r.xs), tile, overlap, W, y0, y1, src.data_ptr(), dtype, src.shape[0], src.shape[1], row0, nd,
+                   float(nodata_out), band.data_ptr(), _stream(gather))
     main.wait_stream(gather)
     if world == 1:
         return band

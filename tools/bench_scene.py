@@ -9,7 +9,14 @@ wrapper (where the scene loop's time goes), ng_scene_tiles / ng_scene_blend kern
 algorithmic bytes against a device-to-device copy measured in the same run, the card's name, power limit and clocks,
 and the `value` of `bench.py --steps K` run right after.
 
+--nodata-frac F adds a swath edge: a corner triangle of area fraction F (legs sqrt(2 F) N, F <= 0.5) set to DN 0 in
+every band of a copy of the scene, predicted with nodata=0.  Recorded besides: the tiles computed and skipped, that
+scene's time and its rate over the computed tiles, the ng_scene_tile_valid time (one tile row of windows, as a host
+scene runs it after each row's copy, and the whole scene in one launch), and nodata=0 against nodata=None on the fully
+valid scene, alternated scene by scene, which shows the cost of the validity pass.
+
     python tools/bench_scene.py --out profiles/scene_bench.json
+    python tools/bench_scene.py --nodata-frac 0.4 --out profiles/scene_bench_nodata.json
 """
 from __future__ import annotations
 
@@ -49,6 +56,83 @@ def event_ms(fn, reps):
     return a.elapsed_time(b) / reps
 
 
+def nodata_section(frac, scene, one_scene, model, emb, sdev, tiles, N, T, ov, B, args, copy_gbs):
+    import math
+    from nirgan_b200 import _lib as L
+    from nirgan_b200 import scene as S
+
+    dev = sdev.device
+    n = len(tiles)
+    i = torch.arange(N, dtype=torch.int32)
+    edge = math.sqrt(2 * frac) * N
+    mask = (i[:, None] + i[None, :]) < edge                  # pixels (y, x) with y + x < sqrt(2 F) N: the swath edge
+    swath = scene.clone().pin_memory()
+    swath.view(torch.int16).masked_fill_(mask, 0)
+    ys, xs = S.scene_grid(N, N, T, ov)
+    nx = len(xs)
+
+    def swath_scene():
+        return S.predict_scene(model, swath, tile=T, overlap=ov, batch_size=B, embeds=emb, nodata=0)
+
+    for _ in range(args.warmup):
+        swath_scene()
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    for _ in range(args.scenes):
+        out = swath_scene()
+    torch.cuda.synchronize()
+    s = (time.perf_counter() - t0) / args.scenes
+    nan = torch.isnan(out[0])
+    mask_ok = bool(torch.equal(nan, mask.to(dev)))
+
+    # nodata=0 against nodata=None on the fully valid scene, alternated scene by scene
+    def valid_scene():
+        return S.predict_scene(model, scene, tile=T, overlap=ov, batch_size=B, embeds=emb, nodata=0)
+
+    valid_scene()
+    times = {"none": [], "nodata0": []}
+    for _ in range(args.scenes):
+        for key, fn in (("none", one_scene), ("nodata0", valid_scene)):
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            o = fn()
+            torch.cuda.synchronize()
+            times[key].append(time.perf_counter() - t0)
+    masked_pixels = int(torch.isnan(o).sum())
+
+    # ng_scene_tile_valid alone on the swath scene: one tile row of windows (a host scene's launch), and the whole
+    # scene in one launch (its counts give the skipped tiles)
+    st = torch.cuda.current_stream().cuda_stream
+    swd = swath.view(torch.int16).to(dev)
+    org = torch.tensor(tiles, dtype=torch.int32, device=dev)
+    cnt = torch.empty(n, dtype=torch.int32, device=dev)
+    row_ms = event_ms(lambda: L.call("ng_scene_tile_valid", swd.data_ptr(), L.U16, 3, N, N, 0, org.data_ptr(), nx, T,
+                                     0.0, cnt.data_ptr(), st), 200)
+    all_ms = event_ms(lambda: L.call("ng_scene_tile_valid", swd.data_ptr(), L.U16, 3, N, N, 0, org.data_ptr(), n, T,
+                                     0.0, cnt.data_ptr(), st), 20)
+    skipped = int((cnt == 0).sum())
+    skipped_grid = sum(1 for y, x in tiles if (y + T - 1) + (x + T - 1) < edge)
+    del swd
+    row_bytes = nx * (3 * T * T * 2 + 4)
+    all_bytes = n * (3 * T * T * 2 + 4)
+    med = {k: sorted(v)[len(v) // 2] for k, v in times.items()}
+    return {
+        "nodata_frac": frac, "triangle_legs_px": edge, "nodata_pixel_frac": float(mask.float().mean()),
+        "tiles": n, "tiles_skipped": skipped, "tiles_computed": n - skipped, "tiles_skipped_by_grid_arithmetic": skipped_grid,
+        "scene_s": s, "computed_tiles_per_s": (n - skipped) / s, "output_mask_equals_triangle": mask_ok,
+        "valid_output_finite": bool(torch.isfinite(out[0][~nan]).all()),
+        "ab_fully_valid_scene": {"scene_s_nodata_none": times["none"], "scene_s_nodata_0": times["nodata0"],
+                                 "median_none": med["none"], "median_nodata_0": med["nodata0"],
+                                 "median_ratio": med["nodata0"] / med["none"], "pixels_masked": masked_pixels},
+        "ng_scene_tile_valid": {
+            "tile_row": {"windows": nx, "ms": row_ms, "bytes": row_bytes, "gbs": row_bytes / row_ms / 1e6,
+                         "frac_of_copy_peak": row_bytes / row_ms / 1e6 / copy_gbs, "ms_per_scene": row_ms * n / nx,
+                         "note": "one tile row's 12.6 MB of scene rows stays in the L2, as right after its copy"},
+            "whole_scene": {"windows": n, "ms": all_ms, "bytes": all_bytes, "gbs": all_bytes / all_ms / 1e6,
+                            "frac_of_copy_peak": all_bytes / all_ms / 1e6 / copy_gbs}},
+    }
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--size", type=int, default=8192)
@@ -58,8 +142,11 @@ def main():
     ap.add_argument("--scenes", type=int, default=4)
     ap.add_argument("--warmup", type=int, default=1)
     ap.add_argument("--bench-steps", type=int, default=20)
+    ap.add_argument("--nodata-frac", type=float, default=None)
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
+    if args.nodata_frac is not None and not 0 < args.nodata_frac <= 0.5:
+        raise SystemExit("bench_scene.py: --nodata-frac must lie in (0, 0.5] (a corner triangle)")
     if not torch.cuda.is_available():
         raise SystemExit("bench_scene.py: no CUDA device")
     import nirgan_b200  # noqa: F401
@@ -133,6 +220,10 @@ def main():
     copy_ms = event_ms(lambda: big2.copy_(big), 10)
     copy_gbs = 2 * big.numel() * 4 / copy_ms / 1e6
     h2d_bytes = scene.numel() * 2
+    nodata_rec = None
+    if args.nodata_frac is not None:
+        nodata_rec = nodata_section(args.nodata_frac, scene, one_scene, model, emb, sdev, tiles, N, T, ov, B, args,
+                                    copy_gbs)
     info = gpu_info()
     del pred, band, big, big2, sdev
     torch.cuda.empty_cache()
@@ -166,6 +257,8 @@ def main():
         "scene_over_bench_value": tps / bench_value if bench_value else None,
         "scene_over_generator_alone": tps / gen_tps,
     }
+    if nodata_rec is not None:
+        rec["nodata"] = nodata_rec
     if r.returncode != 0:
         rec["bench_py"]["stderr_tail"] = r.stderr[-2000:]
     txt = json.dumps(rec, indent=1)
