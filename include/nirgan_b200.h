@@ -48,7 +48,7 @@
  *   ng_image_metrics   utils/calculate_metrics.py:6-37 (L1, L2, PSNR, SSIM)
  *   ng_resize_plane / ng_hist_match / ng_sort_segments
  *                      F.interpolate + skimage.exposure.match_histograms, create_synthetic_dataset.py:34-52,111-118
- *   ng_scene_tiles / ng_scene_blend / ng_scene_tile_valid / ng_scene_blend_masked
+ *   ng_scene_tiles / ng_scene_blend / ng_scene_tile_valid / ng_scene_blend_masked / ng_scene_blend_indices
  *                      the per-tile `model(hr)` loop of create_synthetic_dataset.py:100-118 over pre-cut files plus the
  *                      cutting and stitching a user writes around it for a whole scene (the reference has neither)
  *   ng_satclip_encode  SatClIP_wrapper.predict model/satclip/satclip_wrapper.py:29-34 (location_encoder.py:73-151,
@@ -387,6 +387,18 @@ int ng_scene_blend_masked(const float* pred, const int32_t* slot, const int32_t*
                           int32_t nx, int32_t T, int32_t overlap, int32_t W, int32_t y0, int32_t y1, const void* scene,
                           int32_t dtype, int32_t C, int32_t rows, int32_t row0, float nodata, float nodata_out,
                           float* out, void* stream);
+/* ng_scene_blend (slot NULL) or ng_scene_blend_masked (slot given), followed by k index bands:
+ * out [1 + k][y1-y0][W] fp32 (16-byte aligned when W % 4 == 0), plane 0 the blended NIR, bit-identical to what those
+ * entry points give, plane 1 + i index which[i] (host int32 [k], 1 <= k <= 6, values 1..6: NDVI, NDWI, GNDVI, SAVI,
+ * MSAVI, EVI, utils/remote_sensing_indices.py's order) in index mode -- bit-identical to ng_rs_index(loss_eps = 0) of
+ * that NIR.  R, G, B are channels 0, 1, 2 of scene [C][rows][W] (NG_F32 as is, NG_U16 as (float)dn / dn_scale, the
+ * values ng_scene_tiles cuts), which holds scene rows [row0, row0 + rows) and must contain [y0, y1); C >= 3.  With
+ * use_nodata != 0 a nodata pixel (rule above) is nodata_out in every plane, without it no pixel is masked (slot may
+ * still be given).  Each element is written once. */
+int ng_scene_blend_indices(const float* pred, const int32_t* slot, const int32_t* oy, int32_t ny, const int32_t* ox,
+                           int32_t nx, int32_t T, int32_t overlap, int32_t W, int32_t y0, int32_t y1, const void* scene,
+                           int32_t dtype, int32_t C, int32_t rows, int32_t row0, float dn_scale, int32_t use_nodata,
+                           float nodata, float nodata_out, const int32_t* which, int32_t k, float* out, void* stream);
 
 /* Optional generator losses (utils/losses.py:10-29 ssim_loss, :64-78 emd_loss -- pix2pix.py:12-13,233-242), forward and
  * d/dpred (dpred may be NULL).  ssim_loss: out1[0] = 1 - mean(kornia.metrics.ssim(pred, target, window)); planes = B*C;

@@ -86,6 +86,8 @@ _SIGNATURES = {
     "ng_scene_tile_valid": (c_i32, [c_vp, c_i32, c_i32, c_i32, c_i32, c_i32, c_vp, c_i32, c_i32, c_f32, c_vp, c_vp]),
     "ng_scene_blend_masked": (c_i32, [c_vp, c_vp, c_vp, c_i32, c_vp, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_vp, c_i32,
                                       c_i32, c_i32, c_i32, c_f32, c_f32, c_vp, c_vp]),
+    "ng_scene_blend_indices": (c_i32, [c_vp, c_vp, c_vp, c_i32, c_vp, c_i32, c_i32, c_i32, c_i32, c_i32, c_i32, c_vp,
+                                       c_i32, c_i32, c_i32, c_i32, c_f32, c_i32, c_f32, c_f32, c_vp, c_i32, c_vp, c_vp]),
     "ng_satclip_encode": (c_i32, [c_vp, c_i32, c_i32, c_vp, c_i32, c_i32, c_i32, C.c_double, C.c_double, c_vp, c_vp]),
     "ng_linear": (c_i32, [c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_vp, c_vp]),
     "ng_lsgan_loss": (c_i32, [c_vp, c_i64, c_f32, c_vp, c_i32, c_vp, c_f32, c_vp]),

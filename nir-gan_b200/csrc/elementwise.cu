@@ -3,6 +3,7 @@
 // pixel losses and Adam.  All are vectorised (16-byte accesses on the 16-bit paths) and sized in
 // multiples of the SM count.
 #include "common.cuh"
+#include "rs_index.cuh"
 #include <stdlib.h>
 #include <type_traits>
 
@@ -670,36 +671,8 @@ __global__ void reduce_partials_kernel(const float* __restrict__ partial, int nb
 // term order: 0 = L1(pred, nir), 1 = NDVI, 2 = NDWI, 3 = GNDVI, 4 = SAVI, 5 = MSAVI, 6 = EVI (the reference's iteration
 // order, :45-52).  `mask` selects the terms to evaluate (the kernel is ALU-bound once all six indices are on);
 // criterion 0 = l1 (F.l1_loss), 1 = l2 (F.mse_loss) for the six indices.  Also writes
-// dpred = d( sum_i w_i * term_i ) / dpred.
+// dpred = d( sum_i w_i * term_i ) / dpred.  The per-pixel formulas (RsPix, rs_ndvi ..) are in rs_index.cuh.
 // ---------------------------------------------------------------------------------------------
-struct RsPix {
-  float it, ip, dip;     // index of the target, of the prediction, d(index of the prediction)/dpred
-};
-__device__ __forceinline__ RsPix rs_ndvi(float t, float p, float band, float eps) {
-  const float dp = p + band + eps;
-  return {(t - band) / (t + band + eps), (p - band) / dp, (2.f * band + eps) / (dp * dp)};
-}
-__device__ __forceinline__ RsPix rs_gndvi(float t, float p, float R, float G) {
-  // (n - G) / (ndvi(n) + G) with ndvi(n) = (n - R) / (n + R), no epsilon (remote_sensing_indices.py:169-176)
-  const float ndt = (t - R) / (t + R), ndp = (p - R) / (p + R);
-  const float dnd = 2.f * R / ((p + R) * (p + R));
-  const float den = ndp + G;
-  return {(t - G) / (ndt + G), (p - G) / den, (den - (p - G) * dnd) / (den * den)};
-}
-__device__ __forceinline__ RsPix rs_savi(float t, float p, float R) {
-  const float dp = p + R + 0.5f;
-  return {1.5f * (t - R) / (t + R + 0.5f), 1.5f * (p - R) / dp, 1.5f * (2.f * R + 0.5f) / (dp * dp)};
-}
-__device__ __forceinline__ RsPix rs_msavi(float t, float p, float R) {
-  const float st = sqrtf((2.f * t + 1.f) * (2.f * t + 1.f) - 8.f * (t - R));
-  const float sp = sqrtf((2.f * p + 1.f) * (2.f * p + 1.f) - 8.f * (p - R));
-  return {(2.f * t + 1.f - st) / 2.f, (2.f * p + 1.f - sp) / 2.f, 1.f - (2.f * p - 1.f) / sp};
-}
-__device__ __forceinline__ RsPix rs_evi(float t, float p, float R, float Bl, float eps) {
-  const float k = (R - 7.5f) * (Bl + 1.f);
-  const float dt = (t + 6.f) * k + eps, dp = (p + 6.f) * k + eps;
-  return {2.5f * ((t - R) / dt), 2.5f * ((p - R) / dp), 2.5f * (k * (6.f + R) + eps) / (dp * dp)};
-}
 __device__ __forceinline__ float sgn(float v) { return v > 0.f ? 1.f : (v < 0.f ? -1.f : 0.f); }
 
 struct RsWeights { float w[7]; };

@@ -7,11 +7,16 @@
 // ng_scene_tile_valid counts the valid pixels of each window so that the host can skip windows without one;
 // ng_scene_blend_masked blends a compacted prediction buffer and writes nodata pixels as a fill value.
 //
+// Index bands: ng_scene_blend_indices also writes, after the NIR plane, index-mode RemoteSensingIndices planes (epsilon
+// 0, the formulas of rs_index.cuh that ng_rs_index evaluates) of each pixel's blended NIR and its R, G, B (channels 0-2
+// of the resident scene rows, converted as ng_scene_tiles converts them); nodata pixels are the fill value in every plane.
+//
 // Blend (nirgan_b200/scene.py states the same definitions):
 //   out(y, x) = sum_t w_t(y, x) p_t(y, x) / sum_t w_t(y, x)   over the tiles t covering (y, x), ascending (k_y, k_x)
 //   w(i, j)   = w1(i) w1(j),   w1(i) = min(i + 1, T - i, overlap + 1) / (overlap + 1)
 // computed with the integer weights (overlap + 1)^2 w(i, j), and a pixel covered by a single tile takes that tile's value unchanged.
 #include "common.cuh"
+#include "rs_index.cuh"
 
 namespace ng {
 
@@ -96,12 +101,38 @@ scene_valid_kernel(const E* __restrict__ scene, int C, int rows, int W, int row0
   }
 }
 
-// the nodata mask of the masked blend: scene rows [row0, row0 + rows) resident as scene [C][rows][W]
+// the scene rows the blend reads (the nodata mask, the R, G, B of the index bands): scene rows [row0, row0 + rows)
+// resident as scene [C][rows][W]
 template <typename E> struct SceneMask {
   const E* scene;
   int C, rows, row0;
   float nodata, nodata_out;
 };
+
+// the index bands: which[0 .. k) in RS_TERMS numbering (1 = NDVI .. 6 = EVI), plane 1 + i is index which[i]
+constexpr int SCENE_MAX_INDICES = 6;
+struct SceneIndices {
+  int which[SCENE_MAX_INDICES];
+  int k;
+  float dn_scale;
+};
+
+// index mode of RemoteSensingIndices (epsilon 0) at one pixel of NIR n: the prediction map of ng_rs_index
+__device__ __forceinline__ float rs_index_value(int which, float n, float R, float G, float Bl) {
+  switch (which) {
+    case 1: return rs_ndvi(n, n, R, 0.f).ip;
+    case 2: return rs_ndvi(n, n, G, 0.f).ip;
+    case 3: return rs_gndvi(n, n, R, G).ip;
+    case 4: return rs_savi(n, n, R).ip;
+    case 5: return rs_msavi(n, n, R).ip;
+    default: return rs_evi(n, n, R, Bl, 0.f).ip;
+  }
+}
+
+template <int V> __device__ __forceinline__ void store_px(float* o, const float (&v)[V]) {
+  if constexpr (V == 4) *reinterpret_cast<float4*>(o) = make_float4(v[0], v[1], v[2], v[3]);
+  else *o = v[0];
+}
 
 // (overlap + 1) * w1(i): the common factor cancels in the normalised sum, and the integer weights and their sums are
 // exact in fp32 (at most (overlap + 1)^2 per tile)
@@ -147,13 +178,15 @@ __device__ __forceinline__ float blend_pixel(const float* __restrict__ pred, con
 }
 
 // gather form: every output pixel of rows [y0, y0 + rows) reads its covering tiles and is written once.  V consecutive
-// pixels of one row per thread (V = 4 when W % 4 == 0: one 16-byte store).  MASK: pred is compacted through slot, and
-// a nodata pixel of the resident scene rows is written as mask.nodata_out without reading any prediction.
-template <int V, bool MASK = false, typename E = float>
+// pixels of one row per thread (V = 4 when W % 4 == 0: one 16-byte store per plane).  SLOT: pred is compacted through
+// slot.  MASK: a nodata pixel of the resident scene rows is written as mask.nodata_out without reading any prediction.
+// INDEX: planes 1 .. idx.k (plane p at out + p * rows * W) get the index bands; the R, G, B loads serve the nodata test
+// too.
+template <int V, bool SLOT, bool MASK, bool INDEX, typename E = float>
 __global__ void __launch_bounds__(SC_THREADS)
 scene_blend_kernel(const float* __restrict__ pred, const int* __restrict__ slot, const int* __restrict__ oy, int ny,
                    const int* __restrict__ ox, int nx, int T, int overlap, int W, int y0, int rows, SceneMask<E> mask,
-                   float* __restrict__ out) {
+                   float* __restrict__ out, SceneIndices idx) {
   const int x = (blockIdx.x * blockDim.x + threadIdx.x) * V;
   if (x >= W) return;
   const int ov1 = overlap + 1;
@@ -161,32 +194,77 @@ scene_blend_kernel(const float* __restrict__ pred, const int* __restrict__ slot,
     const int y = y0 + row;
     const int ky0 = first_cover(oy, ny, T, y);
     float* o = out + (size_t)row * W + x;
-    auto px = [&](int xx) -> float {
-      if constexpr (MASK) {
-        const E* srow = mask.scene + (size_t)(y - mask.row0) * W;
-        if (!pixel_valid<E>(srow, mask.C, (size_t)mask.rows * W, xx, mask.nodata)) return mask.nodata_out;
+    if constexpr (INDEX) {
+      const size_t plane = (size_t)mask.rows * W;
+      const E* s = mask.scene + (size_t)(y - mask.row0) * W + x;
+      bool valid[V];
+      float nir[V], R[V], G[V], Bl[V];
+#pragma unroll
+      for (int q = 0; q < V; ++q) {
+        const E r = s[q], g = s[plane + q], b = s[2 * plane + q];
+        valid[q] = true;
+        if constexpr (MASK) {
+          valid[q] = !is_nodata<E>(r, mask.nodata) | !is_nodata<E>(g, mask.nodata) | !is_nodata<E>(b, mask.nodata);
+          for (int c = 3; c < mask.C; ++c) valid[q] |= !is_nodata<E>(s[(size_t)c * plane + q], mask.nodata);
+        }
+        nir[q] = valid[q] ? blend_pixel<SLOT>(pred, slot, oy, ny, ky0, ox, nx, T, ov1, y, x + q) : mask.nodata_out;
+        R[q] = scene_value<E>(r, idx.dn_scale);
+        G[q] = scene_value<E>(g, idx.dn_scale);
+        Bl[q] = scene_value<E>(b, idx.dn_scale);
       }
-      return blend_pixel<MASK>(pred, slot, oy, ny, ky0, ox, nx, T, ov1, y, xx);
-    };
-    if constexpr (V == 4)
-      *reinterpret_cast<float4*>(o) = make_float4(px(x), px(x + 1), px(x + 2), px(x + 3));
-    else
-      *o = px(x);
+      store_px<V>(o, nir);
+      for (int p = 0; p < idx.k; ++p) {
+        const int which = idx.which[p];
+        float v[V];
+#pragma unroll
+        for (int q = 0; q < V; ++q)
+          v[q] = valid[q] ? rs_index_value(which, nir[q], R[q], G[q], Bl[q]) : mask.nodata_out;
+        store_px<V>(o + (size_t)(1 + p) * rows * W, v);
+      }
+    } else {
+      auto px = [&](int xx) -> float {
+        if constexpr (MASK) {
+          const E* srow = mask.scene + (size_t)(y - mask.row0) * W;
+          if (!pixel_valid<E>(srow, mask.C, (size_t)mask.rows * W, xx, mask.nodata)) return mask.nodata_out;
+        }
+        return blend_pixel<SLOT>(pred, slot, oy, ny, ky0, ox, nx, T, ov1, y, xx);
+      };
+      if constexpr (V == 4)
+        *reinterpret_cast<float4*>(o) = make_float4(px(x), px(x + 1), px(x + 2), px(x + 3));
+      else
+        *o = px(x);
+    }
   }
 }
 
-template <bool MASK, typename E>
+template <bool SLOT, bool MASK, bool INDEX, typename E>
 int launch_blend(const float* pred, const int* slot, const int* oy, int ny, const int* ox, int nx, int T, int overlap,
-                 int W, int y0, int y1, SceneMask<E> mask, float* out, void* stream) {
+                 int W, int y0, int y1, SceneMask<E> mask, SceneIndices idx, float* out, void* stream) {
   const bool vec = W % 4 == 0 && ((uintptr_t)out & 15) == 0;
   const int V = vec ? 4 : 1;
   const int per_row = (W + V - 1) / V;
   const dim3 grid((per_row + SC_THREADS - 1) / SC_THREADS, y1 - y0 < 65535 ? y1 - y0 : 65535);
   cudaStream_t st = (cudaStream_t)stream;
-  if (vec) scene_blend_kernel<4, MASK, E><<<grid, SC_THREADS, 0, st>>>(pred, slot, oy, ny, ox, nx, T, overlap, W, y0, y1 - y0, mask, out);
-  else scene_blend_kernel<1, MASK, E><<<grid, SC_THREADS, 0, st>>>(pred, slot, oy, ny, ox, nx, T, overlap, W, y0, y1 - y0, mask, out);
+  if (vec)
+    scene_blend_kernel<4, SLOT, MASK, INDEX, E><<<grid, SC_THREADS, 0, st>>>(pred, slot, oy, ny, ox, nx, T, overlap, W,
+                                                                             y0, y1 - y0, mask, out, idx);
+  else
+    scene_blend_kernel<1, SLOT, MASK, INDEX, E><<<grid, SC_THREADS, 0, st>>>(pred, slot, oy, ny, ox, nx, T, overlap, W,
+                                                                             y0, y1 - y0, mask, out, idx);
   NG_LAUNCH_CHECK("scene_blend_kernel");
   return NG_OK;
+}
+
+// the four (SLOT, MASK) index blends of one element type
+template <typename E>
+int launch_blend_indices(const float* pred, const int* slot, const int* oy, int ny, const int* ox, int nx, int T,
+                         int overlap, int W, int y0, int y1, SceneMask<E> sc, bool masked, SceneIndices idx,
+                         float* out, void* stream) {
+  if (slot)
+    return masked ? launch_blend<true, true, true, E>(pred, slot, oy, ny, ox, nx, T, overlap, W, y0, y1, sc, idx, out, stream)
+                  : launch_blend<true, false, true, E>(pred, slot, oy, ny, ox, nx, T, overlap, W, y0, y1, sc, idx, out, stream);
+  return masked ? launch_blend<false, true, true, E>(pred, slot, oy, ny, ox, nx, T, overlap, W, y0, y1, sc, idx, out, stream)
+                : launch_blend<false, false, true, E>(pred, slot, oy, ny, ox, nx, T, overlap, W, y0, y1, sc, idx, out, stream);
 }
 
 }  // namespace ng
@@ -250,7 +328,8 @@ extern "C" int ng_scene_blend(const float* pred, const int32_t* oy, int32_t ny, 
                               int32_t overlap, int32_t W, int32_t y0, int32_t y1, float* out, void* stream) {
   int r = require_sm100(); if (r) return r;
   r = check_blend(pred, oy, ny, ox, nx, T, overlap, W, y0, y1, out); if (r) return r;
-  return launch_blend<false, float>(pred, nullptr, oy, ny, ox, nx, T, overlap, W, y0, y1, SceneMask<float>{}, out, stream);
+  return launch_blend<false, false, false, float>(pred, nullptr, oy, ny, ox, nx, T, overlap, W, y0, y1, SceneMask<float>{},
+                                                 SceneIndices{}, out, stream);
 }
 
 extern "C" int ng_scene_blend_masked(const float* pred, const int32_t* slot, const int32_t* oy, int32_t ny,
@@ -265,9 +344,46 @@ extern "C" int ng_scene_blend_masked(const float* pred, const int32_t* slot, con
              "scene_blend_masked: rows [%d, %d) are not inside the resident scene rows [%d, %d)", y0, y1, row0,
              row0 + rows);
   if (dtype == NG_F32)
-    return launch_blend<true, float>(pred, slot, oy, ny, ox, nx, T, overlap, W, y0, y1,
-                                     SceneMask<float>{(const float*)scene, C, rows, row0, nodata, nodata_out}, out, stream);
-  return launch_blend<true, uint16_t>(pred, slot, oy, ny, ox, nx, T, overlap, W, y0, y1,
-                                      SceneMask<uint16_t>{(const uint16_t*)scene, C, rows, row0, nodata, nodata_out},
-                                      out, stream);
+    return launch_blend<true, true, false, float>(pred, slot, oy, ny, ox, nx, T, overlap, W, y0, y1,
+                                                  SceneMask<float>{(const float*)scene, C, rows, row0, nodata, nodata_out},
+                                                  SceneIndices{}, out, stream);
+  return launch_blend<true, true, false, uint16_t>(pred, slot, oy, ny, ox, nx, T, overlap, W, y0, y1,
+                                                   SceneMask<uint16_t>{(const uint16_t*)scene, C, rows, row0, nodata,
+                                                                       nodata_out},
+                                                   SceneIndices{}, out, stream);
+}
+
+extern "C" int ng_scene_blend_indices(const float* pred, const int32_t* slot, const int32_t* oy, int32_t ny,
+                                      const int32_t* ox, int32_t nx, int32_t T, int32_t overlap, int32_t W, int32_t y0,
+                                      int32_t y1, const void* scene, int32_t dtype, int32_t C, int32_t rows,
+                                      int32_t row0, float dn_scale, int32_t use_nodata, float nodata, float nodata_out,
+                                      const int32_t* which, int32_t k, float* out, void* stream) {
+  int r = require_sm100(); if (r) return r;
+  r = check_blend(pred, oy, ny, ox, nx, T, overlap, W, y0, y1, out); if (r) return r;
+  NG_REQUIRE(scene && which && rows > 0 && row0 >= 0, NG_E_ARG, "scene_blend_indices: bad arguments");
+  NG_REQUIRE(k >= 1 && k <= SCENE_MAX_INDICES, NG_E_ARG, "scene_blend_indices: k = %d outside [1, %d]", k,
+             SCENE_MAX_INDICES);
+  SceneIndices idx{};
+  for (int i = 0; i < k; ++i) {
+    NG_REQUIRE(which[i] >= 1 && which[i] <= 6, NG_E_ARG, "scene_blend_indices: which[%d] = %d outside [1, 6]", i,
+               which[i]);
+    idx.which[i] = which[i];
+  }
+  idx.k = k;
+  idx.dn_scale = dn_scale;
+  NG_REQUIRE(C >= 3, NG_E_ARG, "scene_blend_indices: the scene has %d channels, the indices need R, G, B", C);
+  NG_REQUIRE(dtype == NG_F32 || dtype == NG_U16, NG_E_ARG, "scene_blend_indices: the scene must be NG_F32 or NG_U16");
+  NG_REQUIRE(dtype != NG_U16 || dn_scale > 0.f, NG_E_ARG, "scene_blend_indices: dn_scale must be positive");
+  NG_REQUIRE(row0 <= y0 && y1 <= row0 + rows, NG_E_SHAPE,
+             "scene_blend_indices: rows [%d, %d) are not inside the resident scene rows [%d, %d)", y0, y1, row0,
+             row0 + rows);
+  NG_REQUIRE(((uintptr_t)out & (W % 4 == 0 ? 15 : 3)) == 0, NG_E_ALIGN,
+             "scene_blend_indices: out must be %d-byte aligned", W % 4 == 0 ? 16 : 4);
+  if (dtype == NG_F32)
+    return launch_blend_indices<float>(pred, slot, oy, ny, ox, nx, T, overlap, W, y0, y1,
+                                       SceneMask<float>{(const float*)scene, C, rows, row0, nodata, nodata_out},
+                                       use_nodata != 0, idx, out, stream);
+  return launch_blend_indices<uint16_t>(pred, slot, oy, ny, ox, nx, T, overlap, W, y0, y1,
+                                        SceneMask<uint16_t>{(const uint16_t*)scene, C, rows, row0, nodata, nodata_out},
+                                        use_nodata != 0, idx, out, stream);
 }

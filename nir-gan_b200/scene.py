@@ -22,13 +22,25 @@ The reference (and ``synth.run_shard``) only runs pre-cut tiles (create_syntheti
   cut, never run, its ``embeds`` row never read.  Nodata pixels come out as ``nodata_out``; every valid pixel is
   bit-identical to ``nodata=None``, because each tile covering it contains it and so is computed: the blend sees the
   same tiles in the same order with the same weights.
+* Index bands (``indices=``, none by default): names from ``INDEX_NAMES`` (``losses.RS_TERMS[1:]``), each at most once.
+  The result gains one plane per name, after the NIR plane and in the caller's order.  Each is the reference's
+  index-mode formula (``RemoteSensingIndices(mode="index")``, ``losses.rs_index(..., loss_eps=False)``: epsilon 0), with
+  ``n`` the blended NIR of plane 0 and ``R, G, B`` channels 0, 1, 2 of the scene exactly as the generator saw them
+  (``dn / dn_scale`` for uint16, the raw value for float32): NDVI ``(n - R)/(n + R)``, NDWI ``(n - G)/(n + G)``, GNDVI
+  ``(n - G)/(ndvi + G)``, SAVI ``1.5 (n - R)/(n + R + 0.5)``, MSAVI ``(2n + 1 - sqrt((2n + 1)^2 - 8 (n - R)))/2``, EVI
+  ``2.5 (n - R)/((n + 6)(R - 7.5)(B + 1))``.  A value the formula makes non-finite (0/0, the square root of a negative)
+  stays so.  Every plane is bit-identical to ``rs_index`` of plane 0; plane 0 is bit-identical to ``indices=()``;
+  nodata pixels are ``nodata_out`` in every plane.  Needs ``input_nc = 3``.
 
 Cutting (``ng_scene_tiles``: conversion + cut in one pass) and blending (``ng_scene_blend``: gather form, every pixel
 written once) are CUDA kernels of ``csrc/scene.cu``; the generator runs through ``Px2Px.forward_async``.  A host scene
 is copied to the device one tile row at a time on a copy stream (through pinned staging when it is not pinned itself),
 so the copy overlaps the generator.  With ``nodata`` the valid pixels of each tile are counted on the device
 (``ng_scene_tile_valid``: once over a device scene, per tile row right after its copy for a host scene), the computed
-tiles are batched in tile-index order, and ``ng_scene_blend_masked`` blends the compacted predictions.
+tiles are batched in tile-index order, and ``ng_scene_blend_masked`` blends the compacted predictions.  With
+``indices`` the blend is ``ng_scene_blend_indices``: the same blend kernel writes the index planes from the NIR value it
+has just computed and the R, G, B of the resident scene rows, which it reads once per pixel for the nodata test too.  The
+band grows to ``(1 + k) (y1 - y0) W`` floats; nothing else grows.
 """
 from __future__ import annotations
 
@@ -38,6 +50,7 @@ from typing import Dict, List, NamedTuple, Optional, Sequence, Tuple
 import torch
 
 from . import _lib as L
+from .losses import RS_TERMS
 
 
 def _check_grid(H: int, W: int, T: int, overlap: int) -> None:
@@ -82,6 +95,25 @@ def band_tile_rows(row_origins: Sequence[int], T: int, y0: int, y1: int) -> Tupl
     """``[k0, k1)``: the tile rows whose rows meet ``[y0, y1)`` (the origins are ascending)."""
     ks = [k for k, o in enumerate(row_origins) if o < y1 and o + T > y0]
     return ks[0], ks[-1] + 1
+
+
+INDEX_NAMES = RS_TERMS[1:]          # ("ndvi", "ndwi", "gndvi", "savi", "msavi", "evi")
+
+
+def _index_ids(indices) -> List[int]:
+    """``RS_TERMS`` numbers (1 = NDVI .. 6 = EVI) of the index names, in the caller's order."""
+    if isinstance(indices, (str, bytes)):
+        raise ValueError(f"indices must be a sequence of index names, not the string {indices!r}")
+    try:
+        names = list(indices)
+    except TypeError:
+        raise ValueError(f"indices must be a sequence of index names, got {indices!r}") from None
+    for v in names:
+        if not isinstance(v, str) or v not in INDEX_NAMES:
+            raise ValueError(f"unknown index {v!r}: indices are names from {INDEX_NAMES}")
+    if len(set(names)) != len(names):
+        raise ValueError(f"indices must not repeat a name, got {tuple(names)}")
+    return [RS_TERMS.index(v) for v in names]
 
 
 def _padding(model) -> int:
@@ -223,13 +255,14 @@ class _Run(NamedTuple):
     stream: torch.cuda.Stream
     slot: Optional[List[int]]     # nodata only: local tile index -> row of pred, -1 for a skipped tile
     mask: Optional[tuple]         # nodata only: (resident scene rows, NG dtype, row0, nodata)
+    rows: Optional[tuple]         # nodata or scene_rows: (resident scene rows, NG dtype, row0), complete on stream
 
 
 @torch.no_grad()
 def _scene_run(model, scene, tile: int, overlap: int, batch_size: int, embeds: Optional[torch.Tensor], dn_scale: float,
-               rank: int, world: int, nodata) -> _Run:
+               rank: int, world: int, nodata, scene_rows: bool = False) -> _Run:
     """Per-tile predictions of ``rank``'s computed tiles (every tile without ``nodata``), complete on ``stream`` and
-    after the event ``done``."""
+    after the event ``done``; with ``nodata`` or ``scene_rows`` the resident scene rows are complete there too."""
     if getattr(model, "concat", False):
         raise NotImplementedError("predict_scene: concat-style SatCLIP generators are not supported")
     if model.training:
@@ -357,15 +390,17 @@ def _scene_run(model, scene, tile: int, overlap: int, batch_size: int, embeds: O
         emb.record_stream(cut)
     if host is not None:
         src.record_stream(cut)
-    mask = None
-    if nd is not None:
+    mask = rows = None
+    if nd is not None or scene_rows:
         if host is not None:
-            gather.wait_event(host.ensure(k1 - 1))    # the blend reads the mask from every resident row
+            gather.wait_event(host.ensure(k1 - 1))    # the blend reads the mask / R, G, B from every resident row
             src.record_stream(gather)
+        rows = (src, dtype, row0)
+    if nd is not None:
         mask = (src, dtype, row0, nd)
     fin = torch.cuda.Event()
     fin.record(gather)
-    return _Run(pred, ys, xs, (k0, k1), (y0, y1), fin, gather, slot, mask)
+    return _Run(pred, ys, xs, (k0, k1), (y0, y1), fin, gather, slot, mask, rows)
 
 
 @torch.no_grad()
@@ -381,8 +416,9 @@ def _scene_predictions(model, scene, tile: int = 256, overlap: int = 32, batch_s
 @torch.no_grad()
 def predict_scene(model, scene, tile: int = 256, overlap: int = 32, batch_size: int = 64,
                   embeds: Optional[torch.Tensor] = None, dn_scale: float = 10000.0, rank: int = 0, world: int = 1,
-                  nodata=None, nodata_out: float = float("nan")):
-    """NIR band of a whole scene (module docstring: grid, blend, bands, nodata).
+                  nodata=None, nodata_out: float = float("nan"), indices: Sequence[str] = ()):
+    """NIR band of a whole scene, and optionally index bands computed from it (module docstring: grid, blend, bands,
+    nodata, index bands).
 
     ``model``: a ``Px2Px`` in eval mode on a CUDA device (plain or SatCLIP-injected; for the latter ``embeds`` is
     ``(n_tiles, 256)`` in tile-index order).  ``scene``: ``(C, H, W)`` float32 reflectance or uint16 digital numbers
@@ -390,22 +426,41 @@ def predict_scene(model, scene, tile: int = 256, overlap: int = 32, batch_size: 
     ``nodata``: ``None`` (every pixel holds data), or the value that marks a nodata pixel in every channel -- an integer
     in [0, 65535] compared with the raw digital numbers of a uint16 scene, any float (NaN included) for a float32 scene.
     Tiles without a valid pixel are skipped (their ``embeds`` rows are never read) and nodata pixels are ``nodata_out``.
-    Returns the ``(1, H, W)`` float32 device tensor for ``world = 1``, else ``(y0, y1, band)`` with ``band`` the
-    ``(1, y1 - y0, W)`` rows of this rank (``gather_bands`` / ``assemble_bands`` put the bands together).  The result
-    is valid on the caller's current stream."""
+    ``indices``: ``k`` distinct names from ``INDEX_NAMES`` = ("ndvi", "ndwi", "gndvi", "savi", "msavi", "evi"); plane
+    ``1 + i`` of the result is index ``indices[i]`` in the reference's index mode (epsilon 0; NDWI ``(n - G)/(n + G)``,
+    GNDVI over ``ndvi + G``, EVI over ``(n + 6)(R - 7.5)(B + 1)``, verbatim), of the pixel's blended NIR ``n`` (plane 0)
+    and its ``R, G, B`` = channels 0-2 as the generator saw them (``dn / dn_scale`` for uint16); a non-finite value of
+    the formula (0/0, MSAVI's square root of a negative) stays as it is, and a nodata pixel is ``nodata_out`` in every
+    plane.  Plane 0 is bit-identical to ``indices=()``, plane ``1 + i`` to ``losses.rs_index(rgb, nir, nir, name,
+    loss_eps=False)[1]`` of it.  Needs ``input_nc = 3``; the default ``()`` runs exactly the NIR-only blend.
+    Returns the ``(1 + k, H, W)`` float32 device tensor for ``world = 1``, else ``(y0, y1, band)`` with ``band`` the
+    ``(1 + k, y1 - y0, W)`` rows of this rank (``gather_bands`` / ``assemble_bands`` put the bands together).  The
+    result is valid on the caller's current stream.  Bad arguments raise ``ValueError`` before any device work."""
     if nodata is not None and (isinstance(nodata_out, bool) or not isinstance(nodata_out, numbers.Real)):
         raise ValueError(f"nodata_out must be a number, got {nodata_out!r}")
-    r = _scene_run(model, scene, tile, overlap, batch_size, embeds, dn_scale, rank, world, nodata)
+    ids = _index_ids(indices)
+    if ids and model.opt.input_nc != 3:
+        raise ValueError(f"index bands need an RGB generator (input_nc = 3: channels 0, 1, 2 are R, G, B), this one "
+                         f"takes input_nc = {model.opt.input_nc}")
+    r = _scene_run(model, scene, tile, overlap, batch_size, embeds, dn_scale, rank, world, nodata, bool(ids))
     (k0, k1), (y0, y1), gather = r.k, r.band, r.stream
     device = r.pred.device
     W = r.xs[-1] + tile
     main = torch.cuda.current_stream(device)
-    band = torch.empty(1, y1 - y0, W, dtype=torch.float32, device=device)
+    band = torch.empty(1 + len(ids), y1 - y0, W, dtype=torch.float32, device=device)
     with torch.cuda.stream(gather):
         oy = torch.tensor(r.ys[k0:k1], dtype=torch.int32).to(device)
         ox = torch.tensor(r.xs, dtype=torch.int32).to(device)
         band.record_stream(gather)
-        if r.mask is None:
+        if ids:
+            src, dtype, row0 = r.rows
+            slot = None if r.slot is None else torch.tensor(r.slot, dtype=torch.int32).to(device)
+            nd = 0.0 if r.mask is None else r.mask[3]
+            L.call("ng_scene_blend_indices", r.pred.data_ptr(), None if slot is None else slot.data_ptr(),
+                   oy.data_ptr(), k1 - k0, ox.data_ptr(), len(r.xs), tile, overlap, W, y0, y1, src.data_ptr(), dtype,
+                   src.shape[0], src.shape[1], row0, float(dn_scale), int(r.mask is not None), nd, float(nodata_out),
+                   (L.c_i32 * len(ids))(*ids), len(ids), band.data_ptr(), _stream(gather))
+        elif r.mask is None:
             L.call("ng_scene_blend", r.pred.data_ptr(), oy.data_ptr(), k1 - k0, ox.data_ptr(), len(r.xs), tile, overlap,
                    W, y0, y1, band.data_ptr(), _stream(gather))
         else:

@@ -15,8 +15,14 @@ scene's time and its rate over the computed tiles, the ng_scene_tile_valid time 
 scene runs it after each row's copy, and the whole scene in one launch), and nodata=0 against nodata=None on the fully
 valid scene, alternated scene by scene, which shows the cost of the validity pass.
 
+--indices ndvi,ndwi,evi (any subset of ndvi, ndwi, gndvi, savi, msavi, evi) adds index bands: the scene with those
+indices against indices=(), alternated scene by scene (medians), and ng_scene_blend_indices against ng_scene_blend on the
+same predictions of the resident scene, with their algorithmic bytes (predictions, plus 2 B per channel and pixel of the
+uint16 scene and (1 + k) 4 B per pixel written for the index blend) against the device-to-device copy.
+
     python tools/bench_scene.py --out profiles/scene_bench.json
     python tools/bench_scene.py --nodata-frac 0.4 --out profiles/scene_bench_nodata.json
+    python tools/bench_scene.py --indices ndvi,ndwi,evi --out profiles/scene_bench_indices.json
 """
 from __future__ import annotations
 
@@ -133,6 +139,49 @@ def nodata_section(frac, scene, one_scene, model, emb, sdev, tiles, N, T, ov, B,
     }
 
 
+def indices_section(names, scene, one_scene, model, emb, sdev, pred, oy, ox, ys, xs, N, T, ov, B, args, copy_gbs,
+                    blend_ms):
+    from nirgan_b200 import _lib as L
+    from nirgan_b200 import scene as S
+
+    def idx_scene():
+        return S.predict_scene(model, scene, tile=T, overlap=ov, batch_size=B, embeds=emb, indices=names)
+
+    idx_scene()
+    times = {"none": [], "indices": []}
+    for _ in range(args.scenes):
+        for key, fn in (("none", one_scene), ("indices", idx_scene)):
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            o = fn()
+            torch.cuda.synchronize()
+            times[key].append(time.perf_counter() - t0)
+            if key == "none":
+                nir = o
+    plane0_same = bool(torch.equal(o[0], nir[0]))
+    del o, nir
+
+    # the blend kernels alone on the same predictions of the resident scene
+    st = torch.cuda.current_stream().cuda_stream
+    k = len(names)
+    which = (L.c_i32 * k)(*[S.INDEX_NAMES.index(n) + 1 for n in names])
+    out = torch.empty(1 + k, N, N, device=sdev.device)
+    idx_ms = event_ms(lambda: L.call("ng_scene_blend_indices", pred.data_ptr(), None, oy.data_ptr(), len(ys),
+                                     ox.data_ptr(), len(xs), T, ov, N, 0, N, sdev.data_ptr(), L.U16, 3, N, 0, 10000.0,
+                                     0, 0.0, 0.0, which, k, out.data_ptr(), st), 10)
+    del out
+    idx_bytes = len(ys) * len(xs) * T * T * 4 + N * N * (3 * 2 + (1 + k) * 4)
+    med = {key: sorted(v)[len(v) // 2] for key, v in times.items()}
+    return {
+        "indices": list(names), "scene_s_indices_none": times["none"], "scene_s_indices": times["indices"],
+        "median_none": med["none"], "median_indices": med["indices"], "median_ratio": med["indices"] / med["none"],
+        "plane0_equals_indices_none": plane0_same,
+        "ng_scene_blend_indices": {"ms_per_scene": idx_ms, "bytes": idx_bytes, "gbs": idx_bytes / idx_ms / 1e6,
+                                   "frac_of_copy_peak": idx_bytes / idx_ms / 1e6 / copy_gbs,
+                                   "over_ng_scene_blend": idx_ms / blend_ms},
+    }
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--size", type=int, default=8192)
@@ -143,8 +192,15 @@ def main():
     ap.add_argument("--warmup", type=int, default=1)
     ap.add_argument("--bench-steps", type=int, default=20)
     ap.add_argument("--nodata-frac", type=float, default=None)
+    ap.add_argument("--indices", default=None)
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
+    names = None
+    if args.indices is not None:
+        names = tuple(v.strip() for v in args.indices.split(",") if v.strip())
+        valid = ("ndvi", "ndwi", "gndvi", "savi", "msavi", "evi")
+        if not names or any(v not in valid for v in names) or len(set(names)) != len(names):
+            raise SystemExit(f"bench_scene.py: --indices takes distinct names from {','.join(valid)}")
     if args.nodata_frac is not None and not 0 < args.nodata_frac <= 0.5:
         raise SystemExit("bench_scene.py: --nodata-frac must lie in (0, 0.5] (a corner triangle)")
     if not torch.cuda.is_available():
@@ -224,6 +280,10 @@ def main():
     if args.nodata_frac is not None:
         nodata_rec = nodata_section(args.nodata_frac, scene, one_scene, model, emb, sdev, tiles, N, T, ov, B, args,
                                     copy_gbs)
+    indices_rec = None
+    if names is not None:
+        indices_rec = indices_section(names, scene, one_scene, model, emb, sdev, pred, oy, ox, ys, xs, N, T, ov, B,
+                                      args, copy_gbs, blend_ms)
     info = gpu_info()
     del pred, band, big, big2, sdev
     torch.cuda.empty_cache()
@@ -259,6 +319,8 @@ def main():
     }
     if nodata_rec is not None:
         rec["nodata"] = nodata_rec
+    if indices_rec is not None:
+        rec["index_bands"] = indices_rec
     if r.returncode != 0:
         rec["bench_py"]["stderr_tail"] = r.stderr[-2000:]
     txt = json.dumps(rec, indent=1)
